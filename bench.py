@@ -12,6 +12,9 @@ copies inside the timed region), roofline of the dominant kernel, cpu_baseline (
 Extra keys: `e2e_lookahead` (the same loop through TorchWrapper(lookahead=True), opt-in), `kernels` (per C-ABI entry point,
 CUDA events, separate pass), `roofline.fp32` when the dominant kernel is the FMA-bound SH-WFS transform.
 Other workloads: --workload cfg1|cfg2|cfg3noise|cfg4|cfg4lowflux|cfg5|cfg5psf|tiny; --policy po4ao runs ConvPolicy rollouts.
+--dump-outputs DIR writes what the last timed step of the device-resident loop returned (obs, reward, Strehl; the last
+rollout step's obs and reward and the reward sums with --policy po4ao) as DIR/<name>.npy.  The environments, atmosphere and
+policy weights are seeded, so the same arguments give the same inputs and two builds can be compared output for output.
 """
 import argparse
 import json
@@ -64,6 +67,30 @@ def oracle_config(nSubap, nLayers, opts=None):
     return AOConfig(**extra, nSubap=nSubap, windSpeed=[float(v) for v in prof["windSpeed"]],
                     windDirection=[float(v) for v in prof["windDirection"]], fractionalR0=prof["fractionalR0"],
                     altitude=[0.0] * nLayers, nZernike=50, nLoop=4096)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, n_envs):
+    """--dump-outputs: writes each of `arrays` (tensors with the environment axis first, or squeezed away when n_envs == 1)
+    as <out_dir>/<name>.npy, float64 kept, everything else as float32.  Past DUMP_LIMIT_BYTES in all, the same fixed seeded
+    sample of environments is taken from every array and its indices are written as env_index.npy."""
+    import numpy as np
+    host = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if hasattr(t, "detach") else np.asarray(t)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        host[name] = a[None] if n_envs == 1 else a
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = max(1, DUMP_LIMIT_BYTES // (total // n_envs + 8))          # + 8: the environment's entry in env_index
+        idx = np.sort(np.random.default_rng(0).choice(n_envs, size=keep, replace=False))
+        host = {name: a[idx] for name, a in host.items()}
+        host["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -375,6 +402,8 @@ def run_gpu_arm(args):
     ms = e0.elapsed_time(e1)
     launches = _lib.launch_count() - l0
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    # copies: the environment keeps the returned tensors as its own state, and reset_soft() below writes into them
+    last_step = {"obs": obs.clone(), "reward": reward.clone(), "strehl": strehl.clone()} if args.dump_outputs else None
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -485,6 +514,8 @@ def run_gpu_arm(args):
         except Exception as ex:          # the baseline must never take the GPU number down with it
             cpu_baseline = {"value": None, "unit": "env-steps/s", "cores": 1, "kind": "port", "sample": f"failed: {ex!r}"}
 
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step, B)
     if rank == 0:
         line = {
             "metric": "closed-loop AO env-steps/sec (batched envs)", "value": value, "unit": "env-steps/s",
@@ -673,14 +704,16 @@ def run_po4ao_arm(args):
     barrier()
     t_wall0 = time.time()
     e0.record()
-    sr, reward_sum, *_ = mbrl.run(env, None, None, None, replay, policy, dynamics, n_history, args.steps, warmup_ts=0, sigma=0.0,
-                                  episode=1, iteration=2, new_screen=False)
+    sr, reward_sum, _, _, obs_last, rewards, _ = mbrl.run(env, None, None, None, replay, policy, dynamics, n_history, args.steps,
+                                                          warmup_ts=0, sigma=0.0, episode=1, iteration=2, new_screen=False)
     e1.record()
     barrier()
     t_wall1 = time.time()
     ms = e0.elapsed_time(e1)
     launches = _lib.launch_count() - l0
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
+    if rank == 0 and args.dump_outputs:          # before the breakdown below steps the environment again
+        dump_outputs(args.dump_outputs, {"obs": obs_last, "reward": rewards[-1], "reward_sum": reward_sum}, B)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -737,7 +770,12 @@ def main():
                     help="pyramid: the papyrus-style environment (SURVEY.md section 8 f-3)")
     ap.add_argument("--policy", default="integrator", choices=["integrator", "po4ao"],
                     help="po4ao: ConvPolicy (n_history 20) rollouts through rlao_b200.PO4AO.mbrl.run with a GPU replay")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them returned (obs, reward, ...; rank 0's environments) "
+                         "as DIR/<name>.npy, at most 64 MB in all; the inputs are seeded, so two builds can be compared")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -8,18 +8,40 @@ MAIN_CODE/integrator_oopao_razor.py:46-70 (generateNewPhaseScreen(17); reset_sof
 env.step(i, action)).  The reference detector seeds its noise from the wall clock (OOPAO/Detector.py:127-130);
 for the noisy fixture the three RandomState attributes are replaced by RandomState(seed), which keeps the
 reference code path untouched and makes its integer frames reproducible.
+
+The OPD and camera-frame snapshots of the trace go to <name>_snapshots.npz beside <name>.npz, so that no fixture file
+grows past 1 MB; load() returns the two as one dictionary.
 """
 import os
 import sys
 
 import numpy as np
 from numpy.random import RandomState
+from threadpoolctl import threadpool_limits
 
 from . import ref_harness as rh
 from .golden_configs import COMPACT, CONFIGS, LITE, STEPS, EPISODE_SEED
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 DET_SEED = 1234
+# BLAS threads the fixtures are recorded and replayed with.  The atmosphere's innovation factor B is the Cholesky factor of
+# a Schur complement formed through pinv of an ill-conditioned covariance: OpenBLAS's thread split alone moves its digest by
+# up to 4e-6 (relative), far above the 1e-7 the oracle is held to, so the split is fixed rather than left to the host.
+BLAS_THREADS = 8
+
+
+def paths(name, golden_dir=OUT):
+    """The fixture of `name`: (<name>.npz, <name>_snapshots.npz)."""
+    return os.path.join(golden_dir, name + ".npz"), os.path.join(golden_dir, name + "_snapshots.npz")
+
+
+def load(name, golden_dir=OUT):
+    """Every array of the fixture of `name`, snapshots included, as one dictionary."""
+    g = {}
+    for path in paths(name, golden_dir):
+        with np.load(path) as z:
+            g.update((k, z[k]) for k in z.files)
+    return g
 
 
 def digest(a):
@@ -111,7 +133,6 @@ def generate(name):
         g["trace_" + k] = v
     g["trace_total"] = env.total[:n].copy()
     g["trace_residual"] = env.residual[:n].copy()
-    g.update(snaps)
     g["snap_steps"] = np.array([n - 1] if name in COMPACT else [0, n // 2, n - 1])
     if lite:
         g["knife_edge"] = np.packbits(knife, axis=1)
@@ -129,13 +150,14 @@ def generate(name):
         g[f"final_buff_{i}"] = ly.buff.copy()
         g[f"final_map_digest_{i}"] = digest(ly.mapShift)
     os.makedirs(OUT, exist_ok=True)
-    path = os.path.join(OUT, name + ".npz")
-    np.savez_compressed(path, **g)
-    print(name, "->", path, os.path.getsize(path) // 1024, "KiB")
+    for path, arrays in zip(paths(name), (g, snaps)):
+        np.savez_compressed(path, **arrays)
+        print(name, "->", path, os.path.getsize(path) // 1024, "KiB")
 
 
 if __name__ == "__main__":
     if not rh.reference_available():
         sys.exit("reference not present: golden fixtures can only be regenerated in the build container")
-    for nm in (sys.argv[1:] or list(CONFIGS)):
-        generate(nm)
+    with threadpool_limits(limits=BLAS_THREADS, user_api="blas"):
+        for nm in (sys.argv[1:] or list(CONFIGS)):
+            generate(nm)

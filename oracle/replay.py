@@ -2,13 +2,20 @@
 same keys, so a test can diff the two dictionaries (TEST INFRASTRUCTURE ONLY)."""
 import numpy as np
 from numpy.random import RandomState
+from threadpoolctl import threadpool_limits
 
 from .ao_oracle import EnvOracle, compute_psf
 from .golden_configs import COMPACT, CONFIGS, STEPS, EPISODE_SEED
-from .make_golden import digest, DET_SEED
+from .make_golden import BLAS_THREADS, digest, DET_SEED
 
 
 def replay_oracle(name, env=None, steps=None):
+    """On the BLAS thread count the fixtures were recorded with, whatever the host's core count."""
+    with threadpool_limits(limits=BLAS_THREADS, user_api="blas"):
+        return _replay_oracle(name, env, steps)
+
+
+def _replay_oracle(name, env, steps):
     cfg = CONFIGS[name]()
     env = env if env is not None else EnvOracle(cfg, detector_seed=DET_SEED)
     g = {}

@@ -12,6 +12,7 @@ import torch
 from oracle.ao_oracle import (AOConfig, ShackHartmannOracle, compute_psf, dm_geometry, dm_modes, flux_map, source_properties,
                               telescope_pupil)
 from oracle.golden_configs import CONFIGS, EPISODE_SEED, STEPS, psf_formula_opd
+from oracle.make_golden import load as load_golden
 from oracle.warp018 import warp_translate
 from parity_util import build_env, new_episode, rel_err
 from rlao_b200 import _lib
@@ -228,7 +229,7 @@ def test_closed_loop_trace_cfg5_vs_reference_golden(dev):
     every step come from the reference's own spots in the fixture; the reconstructor is the GPU-calibrated one, so `obs`
     is compared at the accuracy the two calibrations agree to."""
     cfg = CONFIGS["cfg5"]()
-    gold = np.load(GOLD)
+    gold = load_golden("cfg5")
     env = build_env(cfg, n_envs=1, rng="reference", device=dev)
     assert np.array_equal(env.wfs.valid_subapertures, gold["valid_subapertures"])
     assert np.array_equal(env.dm_mask.astype(bool), gold["validAct"].astype(bool))

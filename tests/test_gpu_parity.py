@@ -11,6 +11,7 @@ import torch
 from oracle.ao_oracle import (AOConfig, AtmosphereOracle, EnvOracle, ShackHartmannOracle, compute_psf,
                               dm_geometry, dm_modes, flux_map, source_properties, telescope_pupil)
 from oracle.golden_configs import CONFIGS, EPISODE_SEED, STEPS
+from oracle.make_golden import load as load_golden
 from oracle.warp018 import warp_translate
 from parity_util import build_env, new_episode, rel_err
 from rlao_b200 import _lib
@@ -393,7 +394,7 @@ def test_dm_surface_vs_oracle_and_linearity(dev):
 # ---------------------------------------------------------------------------------------------------------
 def _trace(name, dev, steps=None):
     cfg = CONFIGS[name]()
-    gold = np.load(os.path.join(os.path.dirname(__file__), "golden", name + ".npz"))
+    gold = load_golden(name)
     env = build_env(cfg, n_envs=1, rng="reference", device=dev)
     orc = EnvOracle(cfg)
     return cfg, gold, env, orc

@@ -1,9 +1,8 @@
 """Pins the CPU oracle (oracle/ao_oracle.py) against fixtures produced by the UNMODIFIED reference
 (tests/golden/*.npz, written by oracle/make_golden.py in the build container)."""
-import os
-
 import numpy as np
 
+from oracle.make_golden import load
 from oracle.replay import replay_oracle
 
 # digests accumulate ~1e3 terms of mixed sign; traces go through a pinv/SVD chain
@@ -11,10 +10,10 @@ RTOL = {"default": 1e-8, "digest": 1e-7}
 
 
 def _check(name, golden_dir):
-    ref = np.load(os.path.join(golden_dir, name + ".npz"))
+    ref = load(name, golden_dir)
     got, _ = replay_oracle(name)
-    assert set(ref.files) == set(got.keys())
-    for k in ref.files:
+    assert set(ref) == set(got)
+    for k in ref:
         a, b = np.asarray(ref[k]), np.asarray(got[k])
         assert a.shape == b.shape, k
         if a.dtype == np.uint8 or a.dtype == bool:
@@ -45,7 +44,7 @@ def test_oracle_matches_reference_noisy_detector_bit_exact(golden_dir):
     """Razor-like detector (photon + read + dark noise, QE, FWC, 10-bit ADC) with the reference's three
     RandomState streams seeded: the integer camera frames must agree exactly."""
     name = "tiny_noise"
-    ref = np.load(os.path.join(golden_dir, name + ".npz"))
+    ref = load(name, golden_dir)
     got, _ = replay_oracle(name)
     for k in ("frame0", "frame_0", f"frame_{ref['snap_steps'][1]}", f"frame_{ref['snap_steps'][2]}"):
         assert np.array_equal(np.asarray(ref[k]).astype(np.int64), np.asarray(got[k]).astype(np.int64)), k
