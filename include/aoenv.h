@@ -319,8 +319,10 @@ int aoenv_dm_rows(const float* coefs, int ldc, const int32_t* act_pos, int nA, i
  * T rows of the surface commanded at the previous step (dm_rows_cur), the camera description of this frame (NULL = ideal),
  * the action [B][nAct2], where the new commands and their T rows go, and the output tensors.  Host time is what this
  * saves: six interpreter-driven calls become one (the step of a single small environment is launch-bound). */
+/* geometric != 0: part 1 runs aoenv_shwfs_geometric instead of aoenv_shwfs_frame_dm + aoenv_shwfs_slopes; `amp` then holds the
+ * flux weights [R][R] (fluxMap, not its square root), and frame / envmax / order / ref_xy / threshold_cog / det are not used. */
 typedef struct {
-  int32_t B, nS, n, nV, lds, nA, nAct, nAct2, ldc, ldr, W, rec_parts, use_tc, reserved;
+  int32_t B, nS, n, nV, lds, nA, nAct, nAct2, ldc, ldr, W, rec_parts, use_tc, geometric;
   float phase_scale, inv_units, threshold_cog, leak;
   double n_pupil;
   const void *pupil, *amp, *valid, *order, *valid_idx, *ref_xy;        /* aoenv_shwfs_frame_dm / aoenv_shwfs_slopes */
@@ -350,6 +352,31 @@ int aoenv_shwfs_measure_f64(const float* opd, const float* pupil, const float* a
                             const int32_t* valid_idx, int nV, const double* ref_xy, double inv_units, double threshold_cog,
                             int F, int nS, int n, double phase_scale, int shared_max, double* frame, uint64_t* envmax,
                             double* slopes, int lds, void* stream);
+
+/* Geometric Shack-Hartmann sensor (ShackHartmann(is_geometric=True); defined in DESIGN.md §2 as the geometric-optics limit of
+ * the diffractive sensor above): per valid lenslet (i, j), the flux-weighted mean over its n x n pixels
+ * [i*n, (i+1)*n) x [j*n, (j+1)*n) of the gradient of the phase (opd_a + second term) * phase_scale, taken as np.gradient
+ * with unit spacing (central differences inside the R x R array, one-sided first differences on its outer rows and columns;
+ * axis 1 -> X, axis 0 -> Y), times inv_units.  No reference is subtracted (a flat wavefront has zero gradient), no detector
+ * runs and no threshold applies.  The OPD terms are the pupil-less ones (OPD_no_pupil): pixels just outside the pupil take
+ * part in the central differences.
+ *   opd_a [B][R][R]; second term: `opd_b` [B][R][R], or `dm` (the separable DM in factored form, as aoenv_shwfs_frame_dm takes
+ *   it; t_rows is not used), or neither.  flux [R][R] = fluxMap (weights); pupil [R][R] (> 0 inside) for the statistics.
+ *   valid_idx [nV]: ascending lenslet numbers i*nS + j of the valid lenslets.  slopes [B][lds]: X block, then Y block
+ *   (= wfs.signal); slope_planes (nullable) [parts][B][lds] bf16, as aoenv_shwfs_slopes writes them; stats (nullable) [B][4]
+ *   float64 with the definition of aoenv_shwfs_frame_dm (with `dm`, the total is centred on the atmosphere's centre value).
+ * One CTA per (environment, strip of lenslet rows): the strip's pixel rows and a one-row halo are staged in shared memory with
+ * 128-bit loads (64-bit when R % 4 != 0), the DM surface is evaluated in registers and never written; slopes are reduced
+ * without atomics (deterministic).  Two launches when stats is given (its reset, then the kernel), else one. */
+int aoenv_shwfs_geometric(const float* opd_a, const float* opd_b, const aoenv_dm_sep_t* dm, const float* pupil,
+                          const float* flux, const int32_t* valid_idx, int nV, int B, int nS, int n, float phase_scale,
+                          float inv_units, float* slopes, int lds, void* slope_planes, int parts, double* stats, void* stream);
+
+/* Calibration-grade twin (init only: slope units, interaction-matrix pushes): the same measurement in float64 arithmetic on
+ * F wavefronts opd [F][R][R] (float32, OPD_no_pupil, metres); slopes [F][lds] float64 = gradient means * phase_scale *
+ * inv_units. */
+int aoenv_shwfs_geometric_f64(const float* opd, const float* flux, const int32_t* valid_idx, int nV, int F, int nS, int n,
+                              double phase_scale, double inv_units, double* slopes, int lds, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Pyramid WFS — OOPAO/Pyramid.py:469-504 (pyramid_transform), :581-603 (modulation), :987-1002 (detector binning)

@@ -4,7 +4,7 @@ parameterFile_oopao_parser.py): `initializeParameterFile(args) -> param` dict.
 
 `args` carries the atmosphere (r0, L0, fractionalR0, windSpeed, windDirection, altitude), nLoop and gainCL as
 in the reference's YAML files, plus optional nSubaperture (default 20), nPixelPerSubap (6), diameter (8),
-magnitude (8), opticalBand ('I'), nZernike (50), noise (False).
+magnitude (8), opticalBand ('I'), nZernike (50), noise (False), is_geometric (False).
 """
 import numpy as np
 
@@ -50,6 +50,7 @@ def initializeParameterFile(args):
     param["lightRatio"] = 0.5
     param["threshold_cog"] = 0.01
     param["shannon_sampling"] = False
+    param["is_geometric"] = bool(g("is_geometric", False))           # geometric sensor (DESIGN.md section 2)
     noisy = bool(g("noise", False))
     param["cam_photonNoise"] = noisy
     param["cam_readoutNoise"] = 14 if noisy else 0                   # OOPAOEnvRazor.py:332-333

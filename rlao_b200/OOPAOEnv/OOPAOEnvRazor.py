@@ -139,7 +139,7 @@ class OOPAO:
                                postProcessing=param.get("postProcessing", "slopesMaps"))
         else:
             self.wfs = ShackHartmann(telescope=self.tel, nSubap=param["nSubaperture"], lightRatio=param.get("lightRatio", 0.5),
-                                     threshold_cog=param.get("threshold_cog", 0.01), is_geometric=False,
+                                     threshold_cog=param.get("threshold_cog", 0.01), is_geometric=param.get("is_geometric", False),
                                      shannon_sampling=param.get("shannon_sampling", True))
         cam = self.wfs.cam
         cam.sensor = param.get("cam_sensor", cam.sensor)
@@ -281,7 +281,7 @@ class OOPAO:
         src = tel.src
         if wfs._flux_version != getattr(src, "_flux_version", 0) or wfs.current_nPhoton != src.nPhoton:
             return None                                   # wfs._measure_terms re-initialises the flux on the ordinary path
-        key = (wfs._flux_version, id(wfs._amp), id(wfs._ref_xy), wfs.slopes_units, wfs.threshold_cog, float(self.leak),
+        key = (wfs._flux_version, wfs.is_geometric, id(wfs._amp), id(wfs._ref_xy), wfs.slopes_units, wfs.threshold_cog, float(self.leak),
                id(self._Rm_op), id(dm._sep), src.wavelength, id(self._coefs_buf))
         if self._native_key == key:
             return self._native
@@ -296,13 +296,19 @@ class OOPAO:
         c.B, c.nS, c.n, c.nV, c.lds = self.n_envs, wfs.nSubap, wfs.n_pix_subap, wfs.nValidSubaperture, wfs._signal.stride(0)
         c.nA, c.nAct, c.nAct2 = dm.nValidAct, dm.nAct, self.nActuator ** 2
         c.ldc, c.ldr, c.W, c.rec_parts, c.use_tc = self._coefs_buf.stride(1), self._rec.stride(0), tables["W"], self._Rm_op.parts, int(tc)
+        c.geometric = int(wfs.is_geometric)
         c.phase_scale, c.inv_units, c.threshold_cog, c.leak = self._phase_scale, 1.0 / wfs.slopes_units, wfs.threshold_cog, self.leak
         c.n_pupil = float(tel.pixelArea)
         keep = [tel._pupil_f, wfs._amp, wfs._valid_u8, wfs._lit_first, wfs._valid_idx, wfs._ref_xy, wfs._frame, wfs._envmax,
                 wfs._stats, wfs._signal, wfs._signal_planes, win, self._Rm, self._Rm_op, self._rec, self._act_idx, self._dm_prev,
                 tables]
         c.pupil, c.amp, c.valid, c.order = tel._pupil_f.data_ptr(), wfs._amp.data_ptr(), wfs._valid_u8.data_ptr(), wfs._lit_first.data_ptr()
-        c.valid_idx, c.ref_xy, c.frame, c.envmax = wfs._valid_idx.data_ptr(), wfs._ref_xy.data_ptr(), wfs._frame.data_ptr(), wfs._envmax.data_ptr()
+        c.valid_idx, c.ref_xy, c.envmax = wfs._valid_idx.data_ptr(), wfs._ref_xy.data_ptr(), wfs._envmax.data_ptr()
+        if wfs.is_geometric:                              # the geometric sensor weighs with the flux and has no frame
+            c.amp, c.frame = wfs._flux.data_ptr(), None
+            keep.append(wfs._flux)
+        else:
+            c.frame = wfs._frame.data_ptr()
         c.stats, c.slopes, c.slope_planes = wfs._stats.data_ptr(), wfs._signal.data_ptr(), wfs._signal_planes.data_ptr()
         c.dm.wlr, c.dm.ilr, c.dm.nActP, c.dm.WL = win[2].data_ptr(), win[1].data_ptr(), dm._rows.shape[2], win[0]
         c.rec_planes = self._Rm_op.planes().data_ptr() if tc else None
@@ -320,7 +326,7 @@ class OOPAO:
         slot = dm._slot
         atm.update()                                                       # :482 (consumes a frame computed ahead)
         self.tel._set_lazy(atm._opd, DMSurfaceRef(dm, slot))               # :488 tel*dm, lazily
-        det = wfs.cam.as_struct(self.env_offset)
+        det = None if wfs.is_geometric else wfs.cam.as_struct(self.env_offset)
         nAct = self.nActuator
         obs = torch.empty((B, nAct, nAct), dtype=torch.float32, device=dev)
         reward = torch.empty((B,), dtype=torch.float32, device=dev)
@@ -360,7 +366,8 @@ class OOPAO:
         self._coefs_slot ^= 1
         dm._coefs, dm._multi, dm._coefs_matrix, dm._slot = coefs, None, None, slot ^ 1
         dm._coefs_of[slot ^ 1], dm._rows_valid[slot ^ 1], dm._valid[slot ^ 1] = coefs, True, False
-        wfs.cam.frame = wfs._frame[0] if B == 1 else wfs._frame
+        if not wfs.is_geometric:
+            wfs.cam.frame = wfs._frame[0] if B == 1 else wfs._frame
         wfs._signal_is_multi = False
         self._obs, self._reward, self._strehl = obs, reward, strehl
         if self.total is not None and i is not None and 0 <= i < self._nLoop:
@@ -569,7 +576,7 @@ class OOPAO:
                                postProcessing=param["postProcessing"])
         elif type == "shackhartmann":
             self.wfs = ShackHartmann(telescope=self.tel, nSubap=param["nSubaperture"], lightRatio=param.get("lightRatio", 0.5),
-                                     threshold_cog=param.get("threshold_cog", 0.01), is_geometric=False,
+                                     threshold_cog=param.get("threshold_cog", 0.01), is_geometric=param.get("is_geometric", False),
                                      shannon_sampling=param.get("shannon_sampling", True))
         else:
             raise NotImplementedError(f"wfs type {type!r}")

@@ -4,6 +4,9 @@
 spots -> detector -> camera frame + per-environment maximum) and aoenv_shwfs_slopes (thresholded centre of
 gravity -> slopes).  Results: `wfs.signal` ([nSignal], or [n_envs, nSignal]; [nSignal, k] after a k-frame
 calibration push as in ShackHartmann.py:674), `wfs.signal_2D`, `wfs.cam.frame`.
+
+`is_geometric=True` builds the geometric sensor instead (DESIGN.md section 2): the flux-weighted mean phase gradient of
+every lenslet, one kernel (aoenv_shwfs_geometric), noise-free; the camera is not used and `wfs.cam.frame` is not written.
 """
 import ctypes as C
 import math
@@ -26,15 +29,13 @@ class ShackHartmann:
         self.telescope = telescope
         if telescope.src is None:
             raise AttributeError("The telescope was not coupled to any source object! Make sure to couple it with an src object using src*tel")
-        if is_geometric:
-            raise NotImplementedError("geometric SH-WFS is out of scope (diffractive path only)")
         if binning_factor != 1 or padding_extension_factor > 2:
             raise NotImplementedError("binning_factor != 1 / extended field of view are out of scope")
         if getattr(telescope.src, "type", "NGS") == "LGS":
             raise NotImplementedError("LGS spot elongation is out of scope")
         self.device = telescope.device
         self.n_envs = telescope.n_envs
-        self._is_geometric = False
+        self._is_geometric = bool(is_geometric)
         self.nSubap = int(nSubap)
         self._lightRatio = lightRatio
         self.binning_factor = 1
@@ -71,7 +72,7 @@ class ShackHartmann:
         # keep_frame = False (default) leaves the camera frame unwritten: `wfs.cam.frame` is then produced on demand from
         # the inputs of the last measurement.
         self.env_offset = 0          # global index of this shard's first environment (seeds of the camera streams)
-        self.use_fused = os.environ.get("AOENV_WFS", "kernels") == "fused"
+        self.use_fused = os.environ.get("AOENV_WFS", "kernels") == "fused" and not self._is_geometric
         self.keep_frame = False
         self._fused_plans = {}
         # inline_dm (default): a separable mirror's surface that exists only as commands (DMSurfaceRef of a lazy mirror) is
@@ -84,7 +85,8 @@ class ShackHartmann:
         self.initialize_flux()
         self._select_valid()
         B = self.n_envs
-        self._frame = torch.zeros((B, R, R), dtype=torch.float32, device=self.device)
+        # (the geometric sensor has no camera frame)
+        self._frame = None if self._is_geometric else torch.zeros((B, R, R), dtype=torch.float32, device=self.device)
         self._envmax = torch.zeros((B,), dtype=torch.int32, device=self.device)
         self._stats = torch.zeros((B, 4), dtype=torch.float64, device=self.device)
         self._signal = torch.zeros((B, self._lds), dtype=torch.float32, device=self.device)
@@ -99,6 +101,8 @@ class ShackHartmann:
         self.photon_per_subaperture = flux.reshape(nS, n, nS, n).sum(axis=(1, 3)).reshape(-1)
         self.photon_per_subaperture_2D = self.photon_per_subaperture.reshape(nS, nS)
         self._amp = torch.as_tensor(np.sqrt(flux), dtype=torch.float32, device=self.device).contiguous()
+        if self._is_geometric:                                           # the weights of the geometric sensor
+            self._flux = torch.as_tensor(flux, dtype=torch.float32, device=self.device).contiguous()
         self.current_nPhoton = src.nPhoton
         self._flux_version = getattr(src, "_flux_version", 0)
         # fused-kernel form: binary pupil mask + one amplitude (valid only when the flux is uniform over the pupil)
@@ -150,8 +154,9 @@ class ShackHartmann:
 
     @is_geometric.setter
     def is_geometric(self, val):
-        if val:
-            raise NotImplementedError("geometric SH-WFS is out of scope")
+        if bool(val) != self._is_geometric:
+            raise NotImplementedError("the calibration (reference, slope units) belongs to the sensor mode: build a new "
+                                      "ShackHartmann(is_geometric=...) instead of switching it")
 
     # ---- kernels ------------------------------------------------------------------------------------------
     def _dm_windows_host(self, dm_tables):
@@ -314,13 +319,10 @@ class ShackHartmann:
                                               C.c_float(self.threshold_cog), F, self.nSubap, self.n_pix_subap,
                                               _lib.ptr(slopes), slopes.stride(0), _lib.ptr(slope_planes), 2, st), "shwfs_slopes")
 
-    def _run(self, opd_a, opd_b, pupil, scale, shared_max, det, frame, envmax, stats, slopes, ref_xy, inv_units,
-             slope_planes=None):
-        lib, st = _lib.load(), _lib.stream_ptr(self.device)
-        F = opd_a.shape[0]
-        dm_struct = None
+    def _second_term(self, opd_b):
+        """(opd_b tensor or None, aoenv_dm_sep_t or None): a separable mirror whose surface exists only as commands is
+        passed in factored form (T = C gx + row windows) and evaluated inside the kernel; any other surface as a tensor."""
         if isinstance(opd_b, DMSurfaceRef):
-            # a separable mirror whose surface exists only as commands: evaluated inside the frame kernel from T = C gx
             tables = opd_b.dm.fused_tables() if (self.inline_dm and opd_b.dm.lazy_surface) else None
             win = self._dm_windows(tables) if tables is not None else None
             if win is not None and not opd_b.materialised:
@@ -328,8 +330,15 @@ class ShackHartmann:
                 dm_struct = _lib.DmSepStruct()
                 dm_struct.rows, dm_struct.wlr, dm_struct.ilr = rows.data_ptr(), win[2].data_ptr(), win[1].data_ptr()
                 dm_struct.nActP, dm_struct.WL, dm_struct.t_rows = rows.shape[1], win[0], 0
-            else:
-                opd_b = opd_b.tensor()
+                return None, dm_struct
+            return opd_b.tensor(), None
+        return opd_b, None
+
+    def _run(self, opd_a, opd_b, pupil, scale, shared_max, det, frame, envmax, stats, slopes, ref_xy, inv_units,
+             slope_planes=None):
+        lib, st = _lib.load(), _lib.stream_ptr(self.device)
+        F = opd_a.shape[0]
+        opd_b, dm_struct = self._second_term(opd_b)
         _lib.check(lib.aoenv_shwfs_frame_dm(_lib.ptr(opd_a), _lib.ptr(opd_b) if dm_struct is None else None,
                                             C.byref(dm_struct) if dm_struct is not None else None, _lib.ptr(self._lit_first),
                                             _lib.ptr(pupil), _lib.ptr(self._amp), _lib.ptr(self._valid_u8), F, self.nSubap,
@@ -341,12 +350,27 @@ class ShackHartmann:
                                           C.c_float(self.threshold_cog), F, self.nSubap, self.n_pix_subap,
                                           _lib.ptr(slopes), slopes.stride(0), _lib.ptr(slope_planes), 2, st), "shwfs_slopes")
 
+    def _run_geometric(self, opd_a, opd_b, slopes, inv_units, slope_planes=None, stats=None):
+        """aoenv_shwfs_geometric: slopes [F, lds] of OPD = opd_a + opd_b (pupil-less), + the pupil statistics."""
+        opd_b, dm_struct = self._second_term(opd_b)
+        _lib.check(_lib.load().aoenv_shwfs_geometric(
+            _lib.ptr(opd_a), _lib.ptr(opd_b), C.byref(dm_struct) if dm_struct is not None else None,
+            _lib.ptr(self.telescope._pupil_f), _lib.ptr(self._flux), _lib.ptr(self._valid_idx), self.nValidSubaperture,
+            opd_a.shape[0], self.nSubap, self.n_pix_subap, C.c_float(2 * math.pi / self.telescope.src.wavelength),
+            C.c_float(inv_units), _lib.ptr(slopes), slopes.stride(0), _lib.ptr(slope_planes), 2, _lib.ptr(stats),
+            _lib.stream_ptr(self.device)), "shwfs_geometric")
+
     def _measure_terms(self, opd_a, opd_b, env_offset=None):
         """Per-environment measurement (single-frame branch, ShackHartmann.py:522-601) on OPD = opd_a + opd_b
         (opd_b: tensor, None, or a DMSurfaceRef = a DM surface that exists only as commands)."""
         if self._flux_version != getattr(self.telescope.src, "_flux_version", 0) or self.current_nPhoton != self.telescope.src.nPhoton:
             self.initialize_flux()                                       # ShackHartmann.py:515-517,534
         tel = self.telescope
+        if self._is_geometric:
+            planes = self._signal_planes if gemm.uses_tensor_cores(opd_a.shape[0]) else None
+            self._run_geometric(opd_a, opd_b, self._signal, 1.0 / self.slopes_units, planes, self._stats)
+            self._signal_is_multi = False
+            return
         env_offset = self.env_offset if env_offset is None else env_offset
         det = self.cam.as_struct(env_offset)
         scale = 2 * math.pi / tel.src.wavelength
@@ -390,10 +414,24 @@ class ShackHartmann:
             _lib.ptr(slopes), lds, _lib.stream_ptr(dev)), "shwfs_measure_f64")
         return slopes
 
+    def _measure_geometric_f64(self, opd, inv_units):
+        """Calibration-grade geometric measurement of F wavefronts [F, R, R] (aoenv_shwfs_geometric_f64).  Returns slopes
+        [F, 2*nValid] float64."""
+        F, nV = opd.shape[0], self.nValidSubaperture
+        slopes = torch.zeros((F, 2 * nV), dtype=torch.float64, device=self.device)
+        opd = opd.to(torch.float32).contiguous()
+        _lib.check(_lib.load().aoenv_shwfs_geometric_f64(
+            _lib.ptr(opd), _lib.ptr(self._flux), _lib.ptr(self._valid_idx), nV, F, self.nSubap, self.n_pix_subap,
+            2 * math.pi / self.telescope.src.wavelength, float(inv_units), _lib.ptr(slopes), 2 * nV,
+            _lib.stream_ptr(self.device)), "shwfs_geometric_f64")
+        return slopes
+
     def measure_frames(self, opd):
         """Multi-frame branch (ShackHartmann.py:605-674): k wavefronts [k, R, R] (OPD_no_pupil, metres), no
         detector, ONE centroiding threshold for the whole batch.  Returns signal [k, nSignal] (float64: this is
         the calibration path)."""
+        if self._is_geometric:                                           # noise-free: the camera is not used
+            return self._measure_geometric_f64(opd, 1.0 / self.slopes_units)
         if self.cam.photonNoise or self.cam.readoutNoise:
             raise NotImplementedError("noisy multi-frame measurements are not supported (calibrate with noise='off')")
         return self._measure_f64(opd, True, self._ref_xy64, 1.0 / self.slopes_units)
@@ -443,12 +481,27 @@ class ShackHartmann:
         self.isInitialized = False
         tel, dev = self.telescope, self.device
         R, nV, nS = tel.resolution, self.nValidSubaperture, self.nSubap
-        lam = tel.src.wavelength
         zero_ref = torch.zeros((2, nV), dtype=torch.float64, device=dev)
+        if self._is_geometric:
+            # a flat wavefront has zero gradient: the reference slopes are exactly zero
+            def centroids(opd):
+                return self._measure_geometric_f64(opd.reshape(1, R, R), 1.0)[0]
+            self._ref_xy64 = zero_ref
+            self._ref_xy = torch.zeros((2, nV), dtype=torch.float32, device=dev)
+            self.reference_slopes_maps = np.zeros((2 * nS, nS))
+        else:
+            def centroids(opd):
+                return self._measure_f64(opd.reshape(1, R, R), False, zero_ref, 1.0)[0]
+            self._init_reference(centroids)
+        self._init_units(centroids)
+        self.isInitialized = True
+        tel.resetOPD()
 
-        def centroids(opd):
-            return self._measure_f64(opd.reshape(1, R, R), False, zero_ref, 1.0)[0]
-
+    def _init_reference(self, centroids):
+        """Reference slopes of the diffractive sensor: the centroids of a flat wavefront."""
+        tel, dev = self.telescope, self.device
+        R, nV, nS = tel.resolution, self.nValidSubaperture, self.nSubap
+        lam = tel.src.wavelength
         flat = centroids(torch.zeros((R, R), dtype=torch.float32, device=dev))
         self._ref_xy64 = flat.reshape(2, nV).contiguous()
         # the float32 step kernels subtract a reference measured by themselves, so that a flat wavefront gives
@@ -469,6 +522,11 @@ class ShackHartmann:
         ref2d[self.validLenslets_x, self.validLenslets_y] = f[:nV]
         ref2d[self.validLenslets_x + nS, self.validLenslets_y] = f[nV:]
         self.reference_slopes_maps = ref2d
+
+    def _init_units(self, centroids):
+        tel, dev = self.telescope, self.device
+        R, nV = tel.resolution, self.nValidSubaperture
+        lam = tel.src.wavelength
         # slope units from five tip ramps.  Quirk kept (ShackHartmann.py:288-290): tel.pupil is an int array, so
         # `Tip[tel.pupil]` fancy-indexes rows 0/1 and the ramp is normalised by the std of the FULL ramp.
         ramp = np.linspace(0, np.pi, R, endpoint=False)
@@ -484,8 +542,6 @@ class ShackHartmann:
             mean_slope[i] = float((c[:nV] - self._ref_xy64[0]).mean())
         self.p = np.polyfit(np.linspace(-2, 2, 5) * amp, mean_slope, deg=1)
         self.slopes_units = float(np.abs(self.p[0]) * (lam / 2 / np.pi))
-        self.isInitialized = True
-        tel.resetOPD()
 
     def __mul__(self, obj):
         """wfs*cam (ShackHartmann.py:769-782): the detector already ran inside the frame kernel."""

@@ -49,7 +49,7 @@ class LayerState(C.Structure):
 class ShStepStruct(C.Structure):
     """aoenv_sh_step_t (include/aoenv.h)."""
     _fields_ = [(k, C.c_int32) for k in ("B", "nS", "n", "nV", "lds", "nA", "nAct", "nAct2", "ldc", "ldr", "W", "rec_parts",
-                                         "use_tc", "reserved")] + [
+                                         "use_tc", "geometric")] + [
         ("phase_scale", C.c_float), ("inv_units", C.c_float), ("threshold_cog", C.c_float), ("leak", C.c_float),
         ("n_pupil", C.c_double)] + [(k, C.c_void_p) for k in ("pupil", "amp", "valid", "order", "valid_idx", "ref_xy", "frame",
                                                               "envmax", "stats", "slopes", "slope_planes")] + [
@@ -96,6 +96,8 @@ PROTOTYPES = {
                           _vp, _vp, _vp],
     "aoenv_shwfs_fused_smem": [_i, _i, _i, _i, _i, _i],
     "aoenv_dm_rows": [_vp, _i, _vp, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp],
+    "aoenv_shwfs_geometric": [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _f, _vp, _i, _vp, _i, _vp, _vp],
+    "aoenv_shwfs_geometric_f64": [_vp, _vp, _vp, _i, _i, _i, _i, _d, _d, _vp, _i, _vp],
     "aoenv_shwfs_measure_f64": [_vp, _vp, _vp, _vp, _vp, _i, _vp, _d, _d, _i, _i, _i, _d, _i, _vp, _vp, _vp, _i, _vp],
     "aoenv_normal_fill": [_u64, _u64, _i, _i, _i, _f, _vp, _vp, _i, _vp],
     "aoenv_vec_to_img": [_vp, _i, _vp, _i, _i, _i, _f, _vp, _vp],

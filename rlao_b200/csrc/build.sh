@@ -3,7 +3,7 @@
 set -euo pipefail
 cd "$(dirname "$0")"
 OUT=${OUT:-../libaoenv_b200.so}
-SRCS="api.cu atm.cu step.cu vk.cu gemm.cu wfs.cu wfs_fused.cu pyr.cu ctrl.cu dm.cu"
+SRCS="api.cu atm.cu step.cu vk.cu gemm.cu wfs.cu wfs_fused.cu wfs_geo.cu pyr.cu ctrl.cu dm.cu"
 [ -f psf.cu ] && SRCS="$SRCS psf.cu"
 [ -f gemm_tc.cu ] && SRCS="$SRCS gemm_tc.cu"
 NVCC=${NVCC:-/usr/local/cuda/bin/nvcc}

@@ -198,7 +198,14 @@ extern "C" int aoenv_sh_step(const aoenv_sh_step_t* c, int parts, const float* o
   AOENV_CHECK_ARG(!(parts & 4) || (action != nullptr && coefs_next != nullptr && dm_rows_next != nullptr), "sh_step: null command argument");
   const bool tc = c->use_tc && c->B > AOENV_SKINNY_MAX_ROWS;
   int rc = 0;
-  if (parts & 1) {                  // spots (DM surface in place) + slopes
+  if ((parts & 1) && c->geometric) {  // geometric slopes (DM surface in place)
+    aoenv_dm_sep_t dm = c->dm;
+    dm.rows = dm_rows_cur;
+    rc = aoenv_shwfs_geometric(opd_a, nullptr, &dm, (const float*)c->pupil, (const float*)c->amp, (const int32_t*)c->valid_idx,
+                               c->nV, c->B, c->nS, c->n, c->phase_scale, c->inv_units, (float*)c->slopes, c->lds,
+                               tc ? c->slope_planes : nullptr, 2, (double*)c->stats, stream);
+    if (rc) return rc;
+  } else if (parts & 1) {           // spots (DM surface in place) + slopes
     aoenv_dm_sep_t dm = c->dm;
     dm.rows = dm_rows_cur;
     rc = aoenv_shwfs_frame_dm(opd_a, nullptr, &dm, (const int32_t*)c->order, (const float*)c->pupil, (const float*)c->amp,
