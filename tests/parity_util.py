@@ -41,6 +41,12 @@ def new_episode(env, seed):
     return env.reset_soft()
 
 
+def knife_edge_lenslets(maps, threshold, margin=1e-4):
+    """Lenslets of `maps` [nValid, n, n] having a pixel within `margin` (relative) of the centroiding `threshold`: the
+    float32 path may legitimately flip such a pixel (SURVEY.md section 7, hard parts)."""
+    return (np.abs(maps - threshold) < margin * threshold).any(axis=(1, 2))
+
+
 def rel_err(a, b):
     a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
     return np.abs(a - b).max() / max(np.abs(b).max(), 1e-300)

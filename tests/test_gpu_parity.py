@@ -13,7 +13,7 @@ from oracle.ao_oracle import (AOConfig, AtmosphereOracle, EnvOracle, ShackHartma
 from oracle.golden_configs import CONFIGS, EPISODE_SEED, STEPS
 from oracle.make_golden import load as load_golden
 from oracle.warp018 import warp_translate
-from parity_util import build_env, new_episode, rel_err
+from parity_util import build_env, knife_edge_lenslets, new_episode, rel_err
 from rlao_b200 import _lib
 
 pytestmark = pytest.mark.gpu
@@ -404,8 +404,7 @@ def _knife_edge_lenslets(orc, margin=1e-4):
     """Valid lenslets of the oracle's last measurement having a pixel within `margin` (relative) of the centroiding
     threshold 0.01 * max: the float32 path may legitimately flip such a pixel (SURVEY.md section 7, hard parts)."""
     maps = orc.wfs.maps_intensity
-    thr = orc.wfs.threshold_cog * maps.max()
-    return (np.abs(maps - thr) < margin * thr).any(axis=(1, 2))
+    return knife_edge_lenslets(maps, orc.wfs.threshold_cog * maps.max(), margin)
 
 
 @pytest.mark.parametrize("name", ["tiny", "cfg1", "cfg3"])
