@@ -2,12 +2,13 @@
 (MAIN_CODE/OOPAOEnv/OOPAOEnv.py:239-249): 4-sided pyramid, PSF centred on four pixels, circular tip-tilt modulation,
 `slopesMaps` post-processing; batched over environments (SURVEY.md section 8 f-3, first step).
 
-The two transforms per modulation point (Pyramid.py:469-504: FFT of the padded field, focal-plane mask, inverse FFT)
-go through cuFFT (`torch.fft`) — the reference's own GPU path does the same through CuPy — over all environments and a
-chunk of modulation points at once; the field formation, mask, intensity accumulation, detector binning and the
-quadrant arithmetic are batched tensor operations around them.  Detector noise uses the camera kernel of the SH path
-(`Detector.integrate` -> aoenv_detector_integrate).  Hand-written transform kernels are future work; parity is pinned
-through oracle/pyramid_oracle.py, itself pinned against the unmodified reference (tests/golden/pyramid.npz).
+The two transforms per modulation point (Pyramid.py:469-504: FFT of the padded field, focal-plane mask, inverse FFT),
+the intensity accumulation over the modulation points and the detector binning run in the library's own kernels
+(aoenv_pyramid_frames, csrc/pyr.cu: hand-written N = 16 x N2 transforms, no cuFFT) for the compiled transform sizes
+(N = 128, 288), over chunks of environments that bound the workspaces.  Other sizes and the float64 calibration frames go
+through `torch.fft`.  The quadrant arithmetic is batched tensor operations.  Detector noise uses the camera kernel of the
+SH path (`Detector.integrate` -> aoenv_detector_integrate).  Parity is pinned through oracle/pyramid_oracle.py, itself
+pinned against the unmodified reference (tests/golden/pyramid.npz).
 Unsupported reference options raise NotImplementedError.
 """
 import math
@@ -183,6 +184,12 @@ class Pyramid:
             self._ktab_key = key
         return self._ktab
 
+    @staticmethod
+    def frames_chunk(nTheta, N, R):
+        """Most environments per aoenv_pyramid_frames call: the workspaces (nTheta transforms of N x R and N x N complex
+        values, one N x N intensity per environment) stay within 2 GiB."""
+        return max(1, (2 << 30) // (nTheta * N * (N + R) * 8 + N * N * 4))
+
     def _frames_kernels(self, opd_a, opd_b):
         """Detector frames [F, n_cam, n_cam] of OPD_no_pupil = opd_a (+ opd_b) through the library's own transform kernels
         (aoenv_pyramid_frames: hand-written N = 16 x N2 FFTs, no cuFFT), environments in chunks that bound the workspaces."""
@@ -190,8 +197,7 @@ class Pyramid:
         R, N, F, dev = tel.resolution, self.nRes, opd_a.shape[0], self.device
         n_cam = self.cam.resolution
         tab = self._kernel_tables()
-        per_env = self.nTheta * N * (N + R) * 8 + N * N * 4
-        chunk = max(1, min(F, (2 << 30) // per_env))
+        chunk = min(F, self.frames_chunk(self.nTheta, N, R))
         ws = getattr(self, "_kernel_ws", None)
         if ws is None or ws[0] != (chunk, self.nTheta):
             ws = ((chunk, self.nTheta), torch.empty((chunk, self.nTheta, N, R, 2), dtype=torch.float32, device=dev),

@@ -47,6 +47,35 @@ def knife_edge_lenslets(maps, threshold, margin=1e-4):
     return (np.abs(maps - threshold) < margin * threshold).any(axis=(1, 2))
 
 
+def psf_window_f64(amp, phase, zeroPaddingFactor, window):
+    """The central `window` x `window` binned pixels of oracle.ao_oracle.compute_psf (even image sizes), as a matrix DFT in
+    float64 on the device of the inputs: amp [R, R], phase [F, R, R] (radians) -> [F, window, window].
+    compute_psf takes fftshift(fft2(ifftshift(sup * phasor))) / N of the field padded to N x N, so output row k is
+    sum_n sup[n] exp(-2 pi i (k - N/2)(n - N/2) / N) / N over the support rows n = pad + y, and the same along x; the
+    half-pixel phasor is applied as the reference rounds it, in complex64."""
+    import torch
+    R = amp.shape[-1]
+    img_res = int(zeroPaddingFactor * R)
+    os_ = 1 if zeroPaddingFactor >= 2 else int(np.ceil(2.0 / zeroPaddingFactor))
+    if os_ % 2 != img_res % 2:
+        os_ += 1
+    N = int(np.fix(zeroPaddingFactor * os_ * R))
+    pad, img_size = int(np.ceil((N - R) / 2)), img_res * os_
+    assert img_res % 2 == 0 and N % 2 == 0 and N == R + 2 * pad and N % 2 == img_size % 2, "even image sizes only"
+    dev = phase.device
+    n = pad + torch.arange(R, device=dev, dtype=torch.int64)
+    phasor = torch.polar(torch.ones(R, R, dtype=torch.float64, device=dev), -np.pi / N * (n[None, :] + n[:, None]).double())
+    field = torch.polar(amp.double().expand_as(phase), phase.double()) * phasor.to(torch.complex64).to(torch.complex128)
+    lo = int(np.ceil(N / 2) - img_size // 2)                       # compute_psf's crop of the image (shift 0: N, img even)
+    c = img_res // 2
+    k = lo + os_ * (c - window // 2) + torch.arange(os_ * window, device=dev, dtype=torch.int64)
+    m = ((k - N // 2)[:, None] * (n - N // 2)[None, :]) % N          # exact integer phase reduction
+    W = torch.polar(torch.ones(m.shape, dtype=torch.float64, device=dev), -2 * np.pi * m.double() / N)
+    emf = W @ field @ W.T / N
+    psf = emf.abs() ** 2
+    return psf.reshape(-1, window, os_, window, os_).sum(dim=(2, 4))
+
+
 def rel_err(a, b):
     a, b = np.asarray(a, dtype=np.float64), np.asarray(b, dtype=np.float64)
     return np.abs(a - b).max() / max(np.abs(b).max(), 1e-300)
