@@ -84,6 +84,20 @@ int aoenv_atm_ring_multi(void* const* wins, const int64_t* win_offsets, void* co
                          int pitch, int64_t env_stride, int nO, const float* X, int ldx, int32_t* flag,
                          int force_rescan, void* stream);
 
+/* Episode reset of a subset of the environments (zero-shift add_row, as after a new screen): the same two steps for the k
+ * environments env_idx [k] (device, int32, distinct, each in [0, B)) of G layers at their windows' CURRENT origin.
+ * Workspace row g*k + j belongs to environment env_idx[j].  The gather reads Z from that environment's window (no shift)
+ * and draws xi from Philox (seeds[g]; counter = ring index, env_idx[j], stream_ids[g]): the caller keys these draws in a
+ * domain of its own, so that they are none of the per-frame add_row draws.  The ring kernel writes row g*k + j of X on
+ * environment env_idx[j]'s window and always rescans its extrema: all three blocks of ext [3][B][2] are exact for the
+ * listed environments afterwards and untouched for the others.  flag: G*k entries. */
+int aoenv_atm_gather_envs(const void* const* wins, const uint64_t* seeds, const uint64_t* stream_ids, int G,
+                          const int32_t* env_idx, int k, int M, int pitch, int64_t env_stride, const int32_t* inner_rc,
+                          int nI, int nO, float* zx, int ldz, void* zx_planes, int parts, void* stream);
+int aoenv_atm_ring_envs(void* const* wins, const int64_t* win_offsets, void* const* exts, int G, const int32_t* env_idx,
+                        int k, int B, int M, int pitch, int64_t env_stride, int nO, const float* X, int ldx, int32_t* flag,
+                        void* stream);
+
 /* Canvas re-centring: copies the window from src_win to dst_win (another canvas buffer, origin 16-byte aligned) and
  * adds pos_delta to the positions stored in ext [3][B][2]. */
 int aoenv_atm_compact(const float* src_win, float* dst_win, int B, int M, int pitch, int64_t env_stride, uint64_t* ext,
@@ -109,6 +123,16 @@ int aoenv_vk_screens(uint64_t seed, uint32_t screen0, int S, int N, const float*
                      const float* h_mx, const float* h_my, void* work_planes, float* work_a, int lda, float* work_b, int ldb,
                      float* dst, int pitch, int64_t env_stride, void* stream);
 
+/* aoenv_vk_screens for a list of environments: screen s is drawn from Philox stream screen0 + env_idx[s] (the stream
+ * aoenv_vk_screens gives environment env_idx[s] when it draws the whole batch from screen0) and written into the window
+ * interior of environment env_idx[s] (dst = row 1, column 1 of environment 0's window).  env_idx [S]: device int32,
+ * distinct.  No injected draws; workspaces as above, sized for S screens. */
+int aoenv_vk_screens_envs(uint64_t seed, uint32_t screen0, const int32_t* env_idx, int S, int N, const float* amp,
+                          const void* wa_planes, const void* wb_planes, int Kp, int parts, const float* sh_ex,
+                          const float* sh_ey, const float* h_amp, const float* h_mx, const float* h_my, void* work_planes,
+                          float* work_a, int lda, float* work_b, int ldb, float* dst, int pitch, int64_t env_stride,
+                          void* stream);
+
 /* updateLayer tail + fill_phase_support + set_OPD (Atmosphere.py:406-407,439-450,474-478): for each layer the
  * bicubic (4x4 tap) sub-pixel shift of the map, clipped to the map's [min,max], cropped to the R x R pupil
  * footprint, weighted by sqrt(fractionalR0) and summed; opd_out [B][R][R] = sum * opd_scale (lambda/2pi).
@@ -121,6 +145,12 @@ int aoenv_atm_phase(const float* const* h_canvas, const uint64_t* const* h_ext, 
                     int R, int M, int Mc, int pitch, int fp_off, const int32_t* h_row_off, const int32_t* h_col_off,
                     const float* h_wrow, const float* h_wcol, const float* h_weight, float opd_scale, float* opd_out,
                     void* stream);
+/* aoenv_atm_phase for the k environments env_idx [k] (device int32, each in [0, B)) of the batch of B: writes their rows of
+ * opd_out [B][R][R] only, with the same per-environment arithmetic (bit for bit what aoenv_atm_phase writes there). */
+int aoenv_atm_phase_envs(const float* const* h_canvas, const uint64_t* const* h_ext, const int32_t* h_org, int nLayer,
+                         int B, int R, int M, int Mc, int pitch, int fp_off, const int32_t* h_row_off,
+                         const int32_t* h_col_off, const float* h_wrow, const float* h_wcol, const float* h_weight,
+                         float opd_scale, const int32_t* env_idx, int k, float* opd_out, void* stream);
 
 /* One frame of Atmosphere.update() (OOPAO/Atmosphere.py:350-428) sequenced on the host side of the library instead of by
  * the Python layer: per layer the add_row steps of this frame (integer part of updateLayer), canvas re-centring, the

@@ -59,7 +59,7 @@ class _LayerView:
     def mapShift(self):
         a = self._atm
         if a._prefetched:                    # a frame computed ahead on the side stream may still be writing the ring
-            torch.cuda.current_stream(a.device).wait_event(a._prefetch_event)
+            a._wait_prefetch()
         oy, ox = a._org[self._i]
         m = a._maps[self._i, a._cur[self._i], :, oy:oy + a._M, ox:ox + a._M]
         return m[0] if a.n_envs == 1 else m
@@ -244,15 +244,24 @@ class Atmosphere:
             if phase is not None:
                 self._maps[i, 0, :, oy + 1:oy + self._M - 1, ox + 1:ox + self._M - 1] = phase
             else:
-                key = (float(self._r0), float(self._L0))
-                if getattr(self, "_synth_key", None) != key:
-                    self._synth, self._synth_key = vk.ScreenSynth(self._r0, self._L0, N, delta, dev), key
-                sseed = (self.seed * 1000003 + screen_seed(i) * 7919 + 12345) & 0xFFFFFFFFFFFFFFFF
                 dst = self._maps[i, 0].data_ptr() + 4 * ((oy + 1) * self._pitch + ox + 1)
-                self._synth.generate(sseed, self.env_offset, B, dst, self._pitch, self._env_stride,
-                                     inject=self.screen_inject[i] if self.screen_inject is not None else None)
+                self._screen_synth().generate(self._screen_key(screen_seed(i)), self.env_offset, B, dst, self._pitch,
+                                              self._env_stride,
+                                              inject=self.screen_inject[i] if self.screen_inject is not None else None)
             self._extrude(i, 0, 0, force_rescan=True)
             ly.notDoneOnce = True
+
+    def _screen_synth(self):
+        key = (float(self._r0), float(self._L0))
+        if getattr(self, "_synth_key", None) != key:
+            ops = self._ops
+            self._synth = vk.ScreenSynth(self._r0, self._L0, ops.layer_res, ops.layer_D / ops.layer_res, self.device)
+            self._synth_key = key
+        return self._synth
+
+    def _screen_key(self, screen_seed):
+        """Philox key of a layer's screens (the stream of environment e is env_offset + e)."""
+        return (self.seed * 1000003 + screen_seed * 7919 + 12345) & 0xFFFFFFFFFFFFFFFF
 
     # ---- device steps -------------------------------------------------------------------------------
     def _fresh_origin(self, i):
@@ -409,8 +418,9 @@ class Atmosphere:
             for k in range(0, len(group), self._group_max):
                 self._extrude_group(group[k:k + self._group_max])
 
-    def _publish(self, out=None):
-        """Sub-pixel shift of every layer + Cn2-weighted sum -> OPD_no_pupil (Atmosphere.py:406-407,439-478)."""
+    def _publish(self, out=None, env_idx=None):
+        """Sub-pixel shift of every layer + Cn2-weighted sum -> OPD_no_pupil (Atmosphere.py:406-407,439-478); with
+        env_idx (int32 device tensor), the rows of those environments only."""
         out = self._opd if out is None else out
         L = self.nLayer
         maps = (C.c_void_p * L)(*[self._maps[i, self._cur[i]].data_ptr() for i in range(L)])
@@ -425,10 +435,13 @@ class Atmosphere:
             for k in range(4):
                 wr[4 * i + k], wc[4 * i + k] = wrow[k], wcol[k]
             wt[i] = math.sqrt(self.fractionalR0[i])
-        _lib.check(_lib.load().aoenv_atm_phase(maps, exts, org, L, self.n_envs, self.telescope.resolution, self._M, self._Mc,
-                                               self._pitch, self._fp_off, roff, coff, wr, wc, wt,
-                                               C.c_float(self.wavelength / 2 / math.pi), _lib.ptr(out),
-                                               _lib.stream_ptr(self.device)), "atm_phase")
+        args = (maps, exts, org, L, self.n_envs, self.telescope.resolution, self._M, self._Mc, self._pitch, self._fp_off, roff,
+                coff, wr, wc, wt, C.c_float(self.wavelength / 2 / math.pi))
+        if env_idx is None:
+            _lib.check(_lib.load().aoenv_atm_phase(*args, _lib.ptr(out), _lib.stream_ptr(self.device)), "atm_phase")
+        else:
+            _lib.check(_lib.load().aoenv_atm_phase_envs(*args, _lib.ptr(env_idx), env_idx.numel(), _lib.ptr(out),
+                                                        _lib.stream_ptr(self.device)), "atm_phase_envs")
 
     def _advance(self, out):
         """One frame: the add_row steps of every layer, then the sub-pixel shift into `out`.  Sequenced by the library
@@ -485,12 +498,17 @@ class Atmosphere:
         self._prefetched = True
         return True
 
+    def _wait_prefetch(self):
+        """Makes the current stream wait for the frame computed ahead (and for what reset_envs changed in it)."""
+        if self._prefetch_event is not None:
+            torch.cuda.current_stream(self.device).wait_event(self._prefetch_event)
+
     def _join_prefetch(self, consume):
         """Makes the current stream wait for a prefetched frame; consume=True makes it the current frame, False drops it
         (the layers have moved on by one frame nobody saw: only for calls that replace the screens anyway)."""
         if not self._prefetched:
             return False
-        torch.cuda.current_stream(self.device).wait_event(self._prefetch_event)
+        self._wait_prefetch()
         self._prefetched = False
         if consume:
             self._opd, self._opd_next = self._opd_next, self._opd
@@ -523,6 +541,96 @@ class Atmosphere:
         self._publish()
         if self.telescope.isPaired:
             self * self.telescope
+
+    # ---- episode reset of a subset of the environments ------------------------------------------------------------
+    RESET_STREAM = 1 << 63          # stream-id bit of the ring innovations of reset_envs: no per-frame add_row sets it
+
+    def env_index(self, env_ids):
+        """Environment list of reset_envs -> sorted, distinct int32 device tensor.  `env_ids`: host list / array of
+        indices, or a bool mask [n_envs] (on the device: counting it costs one synchronisation)."""
+        B = self.n_envs
+        if torch.is_tensor(env_ids) and env_ids.dtype == torch.bool:
+            if tuple(env_ids.shape) != (B,):
+                raise ValueError(f"reset mask of shape {tuple(env_ids.shape)}, expected ({B},)")
+            return torch.nonzero(env_ids.to(self.device)).reshape(-1).to(torch.int32)
+        ids = np.asarray(env_ids.cpu() if torch.is_tensor(env_ids) else env_ids).reshape(-1)
+        if ids.dtype == bool:
+            if ids.shape != (B,):
+                raise ValueError(f"reset mask of shape {ids.shape}, expected ({B},)")
+            ids = np.nonzero(ids)[0]
+        if ids.size and (not np.issubdtype(ids.dtype, np.integer) or ids.min() < 0 or ids.max() >= B):
+            raise ValueError(f"environment indices must be integers in [0, {B})")
+        t = torch.from_numpy(np.unique(ids).astype(np.int32))
+        if self.device.type == "cuda":               # pinned, so that the upload does not synchronise the stream
+            return t.pin_memory().to(self.device, non_blocking=True)
+        return t
+
+    def _check_partial_reset(self):
+        if self.rng != "philox":
+            raise NotImplementedError("reset_envs draws from the counter-based generator: rng='reference' has one host stream "
+                                      "per environment and is not supported")
+        if self.xi_queue is not None or self.xi_log is not None or self.screen_inject is not None:
+            raise NotImplementedError("reset_envs does not support injected or recorded draws (xi_queue / xi_log / screen_inject)")
+        if self.user_defined_opd:
+            raise NotImplementedError("reset_envs redraws the layers: the OPD was set by the user (update(OPD))")
+
+    def reset_envs(self, env_ids, seed):
+        """New episode for the environments `env_ids` only: their windows in every layer get the screen and the outer ring
+        that generateNewPhaseScreen(seed) draws for them, the other environments are untouched bit for bit.
+
+        The reset applies to the frame the next update() returns, whatever the prefetch setting: that frame is computed
+        now if it has not been computed ahead, then the listed environments' windows are redrawn at the layers' current
+        origins and their rows of it are recomputed.  Screen of environment e: the Philox stream generateNewPhaseScreen
+        gives it.  Ring: the zero-shift add_row of a new screen, with innovations keyed by (seed, layer, env_offset + e) in
+        a stream domain of their own (RESET_STREAM): the layers' add_row counters do not move, so every other environment
+        draws exactly what it would have drawn.  The one difference from generateNewPhaseScreen: the sub-pixel phase of the
+        wind (layer.buff) and the window origin belong to the layer, so a reset environment keeps the batch's values, where
+        a full reset sets buff = 0.
+
+        env_ids: host list / array of indices, or a bool mask [n_envs]; a mask on the device costs one synchronisation
+        (to count it).  Returns the int32 device tensor of the reset environments."""
+        self._check_partial_reset()
+        return self._reset_listed(self.env_index(env_ids), seed)
+
+    def _reset_listed(self, idx, seed):
+        """reset_envs for idx = env_index(...)."""
+        k = idx.numel()
+        if k == 0:
+            return idx
+        if self._prefetched:
+            self._wait_prefetch()
+        else:
+            # the frame the next update() returns, through the prefetch machinery (in line on the current stream)
+            if self._opd_next is None:
+                self._opd_next = torch.empty_like(self._opd)
+            self._advance(self._opd_next)
+            self._prefetched = True
+        lib, st, M, pitch, es = _lib.load(), _lib.stream_ptr(self.device), self._M, self._pitch, self._env_stride
+        synth = self._screen_synth()
+        for i in range(self.nLayer):
+            dst = self._win_ptr(i) + 4 * (pitch + 1)                      # window interior, current canvas and origin
+            synth.generate(self._screen_key(seed + i), self.env_offset, k, dst, pitch, es, env_idx=idx)
+        for g0 in range(0, self.nLayer, self._group_max):
+            layers = list(range(g0, min(self.nLayer, g0 + self._group_max)))
+            G = len(layers)
+            tc = gemm.uses_tensor_cores(G * k)
+            wins = (C.c_void_p * G)(*[self._win_ptr(i) for i in layers])
+            seeds = (C.c_uint64 * G)(*[(self.seed * 1000003 + seed + i * 1000) & 0xFFFFFFFFFFFFFFFF for i in layers])
+            ids = (C.c_uint64 * G)(*[self.RESET_STREAM | (self.env_offset << 40) | i for i in layers])
+            _lib.check(lib.aoenv_atm_gather_envs(wins, seeds, ids, G, _lib.ptr(idx), k, M, pitch, es, _lib.ptr(self._inner_rc),
+                                                 self._nI, self._nO, None if tc else _lib.ptr(self._zx), self._K,
+                                                 _lib.ptr(self._zx_planes) if tc else None, self._W_op.parts, st),
+                       "atm_gather_envs")
+            gemm.gemm_tn(self._zx, self._W_op, self._X, G * k, self._nO, backend="tc" if tc else "simt",
+                         x_planes=self._zx_planes if tc else None)
+            offs = (C.c_int64 * G)(*[self._org[i][0] * pitch + self._org[i][1] for i in layers])
+            exts = (C.c_void_p * G)(*[self._ext[i].data_ptr() for i in layers])
+            _lib.check(lib.aoenv_atm_ring_envs(wins, offs, exts, G, _lib.ptr(idx), k, self.n_envs, M, pitch, es, self._nO,
+                                               _lib.ptr(self._X), self._ldx, _lib.ptr(self._flag), st), "atm_ring_envs")
+        self._publish(self._opd_next, env_idx=idx)
+        if self._opd.is_cuda:
+            self._prefetch_event = torch.cuda.current_stream(self.device).record_event()
+        return idx
 
     def __mul__(self, obj):
         """atm*tel / atm*src (Atmosphere.py:632-668).  atm*src points the paired telescope at `src` (which must lie inside
@@ -563,7 +671,7 @@ class Atmosphere:
         self._r0 = val
         if not self.hasNotBeenInitialized:
             if self._prefetched:             # a frame computed ahead (with the old value) may still be reading the operator
-                torch.cuda.current_stream(self.device).wait_event(self._prefetch_event)
+                self._wait_prefetch()
             self.seeingArcsec = 206265 * (self.wavelength / val)
             self._ops.B = self._ops.innovation_factor(val)
             self._upload_B()

@@ -66,6 +66,10 @@ class OOPAO(_RazorOOPAO):
         frame = self.wfs.cam.frame
         return obs, frame.clone(), reward, strehl, done, info
 
+    def reset_envs(self, env_ids, seed):
+        raise NotImplementedError("reset_envs is not available on the Pyramid environment: its science cameras integrate "
+                                  "exposures across steps over the whole batch")
+
     def render4plot(self, current_i):
         """OOPAOEnv.py:473-482: short-exposure PSF of the current residual (log10) and, after the first 15 frames, its
         running mean over the frames rendered so far (the long-exposure product the plots show).  The mean is kept as a

@@ -264,6 +264,36 @@ class OOPAO:
         raise NotImplementedError("reset() rebuilds the whole simulation in the reference (set_params without arguments, "
                                   "OOPAOEnvRazor.py:66-71, which raises there too); use set_params(...) then reset_soft()")
 
+    def reset_envs(self, env_ids, seed):
+        """New episode for the environments `env_ids` only (the others continue bit for bit): new phase screens in every
+        layer (Atmosphere.reset_envs, which applies them to the frame the next step measures) and a flat mirror — their
+        rows of the current commands, of dm_prev, of the current surface's T = C gx rows and, if it is materialised, of
+        the surface itself are zeroed.  The next step's sensor sees the new atmosphere with a flat mirror, and its command
+        is that step's action alone.  No physical parameter is per environment: the operators, wind, r0, L0, the sub-pixel
+        phase of the wind and the window origins stay the batch's (see Atmosphere.reset_envs for the one difference from
+        generateNewPhaseScreen).
+
+        env_ids: host list / array of indices, or a bool mask [n_envs]; a mask on the device costs one synchronisation.
+        Returns the int32 device tensor of the reset environments."""
+        atm, dm = self.atm, self.dm
+        atm._check_partial_reset()
+        idx = atm.env_index(env_ids)
+        if idx.numel() == 0:
+            return idx
+        if dm._coefs_matrix is not None or dm._multi is not None:
+            raise NotImplementedError("reset_envs needs per-environment commands (the mirror holds a calibration command matrix)")
+        atm._reset_listed(idx, seed)
+        rows = idx.long()
+        slot = dm._slot
+        self._dm_prev[rows] = 0
+        for c in {id(t): t for t in (dm._coefs, dm._coefs_of[slot]) if t is not None}.values():
+            c[rows] = 0
+        if dm._rows is not None and dm._rows_valid[slot]:
+            dm._rows[slot][rows] = 0                      # T = C gx: zero commands give exactly zero rows
+        if dm._valid[slot]:
+            dm._opd[slot][rows] = 0
+        return idx
+
     def reset_soft_wfs(self):
         self.action_buffer = []
         return self.wfs.cam.frame.clone()
@@ -456,7 +486,7 @@ class OOPAO:
         atm = self.atm
         nxt = None
         if atm._prefetched:                  # the layers already hold the next frame: keep its OPD with them
-            torch.cuda.current_stream(self.device).wait_event(atm._prefetch_event)
+            atm._wait_prefetch()
             nxt = atm._opd_next.detach().cpu().clone()
         layers = []
         for i, ly in enumerate(atm._layers):

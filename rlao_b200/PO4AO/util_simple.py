@@ -153,6 +153,13 @@ class TorchWrapper(_Wrapper):
             ready.synchronize()            # the caller may reuse its action buffer as soon as step returns
         return cur["bufs"]
 
+    def reset_envs(self, env_ids, seed):
+        """OOPAO.reset_envs of the wrapped environment (not in lookahead mode: its next observation is already measured)."""
+        if self.lookahead:
+            raise NotImplementedError("reset_envs with TorchWrapper(lookahead=True): the next observation has already been "
+                                      "measured from the current episodes")
+        return self._env.reset_envs(env_ids, seed)
+
     def flush(self):
         """Drops the frame measured ahead (lookahead mode): the next step measures again from the current state (the
         atmosphere stays one update ahead)."""

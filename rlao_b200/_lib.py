@@ -76,12 +76,17 @@ PROTOTYPES = {
     "aoenv_atm_ring": [_vp, _i, _i, _i, _i64, _i64, _i, _vp, _i, _vp, _vp, _i, _vp],
     "aoenv_atm_gather_multi": [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i64, _vp, _i, _i, _vp, _vp, _i, _vp, _i, _vp],
     "aoenv_atm_ring_multi": [_vp, _vp, _vp, _i, _i, _i, _i, _i64, _i, _vp, _i, _vp, _i, _vp],
+    "aoenv_atm_gather_envs": [_vp, _vp, _vp, _i, _vp, _i, _i, _i, _i64, _vp, _i, _i, _vp, _i, _vp, _i, _vp],
+    "aoenv_atm_ring_envs": [_vp, _vp, _vp, _i, _vp, _i, _i, _i, _i, _i64, _i, _vp, _i, _vp, _vp],
     "aoenv_atm_compact": [_vp, _vp, _i, _i, _i, _i64, _vp, _i64, _vp],
     "aoenv_vk_screens": [_u64, C.c_uint32, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i,
                          _vp, _i, _i64, _vp],
+    "aoenv_vk_screens_envs": [_u64, C.c_uint32, _vp, _i, _i, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp,
+                              _i, _vp, _i, _i64, _vp],
     "aoenv_atm_update": [_vp, _vp, _vp, _vp],
     "aoenv_sh_step": [_vp, _i] + [_vp] * 12,
     "aoenv_atm_phase": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _vp],
+    "aoenv_atm_phase_envs": [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _f, _vp, _i, _vp, _vp],
     "aoenv_gemm_tn": [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _f, _vp],
     "aoenv_split_bf16": [_vp, _i, _i, _i, _i, _vp, _i, _vp],
     "aoenv_gemm_tn_tc": [_vp, _vp, _i, _i, _vp, _i, _i, _i, _i, _f, _vp],

@@ -25,20 +25,25 @@ struct AtmGroup {
   int sx[AOENV_MAX_LAYERS], sy[AOENV_MAX_LAYERS];
 };
 
+// kEnvs: workspace row b belongs to environment env_idx[b] (the episode reset of a subset, aoenv_atm_gather_envs); the
+// environment index is also the Philox counter word, so a row's innovation does not depend on which others are listed.
+template <bool kEnvs>
 __global__ void __launch_bounds__(256)
 atm_gather_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t env_stride,
                   const int2* __restrict__ inner_rc, int nI, int nO, const float* __restrict__ xi,
-                  float* __restrict__ zx, int ldz, __nv_bfloat16* __restrict__ planes, int parts) {
+                  float* __restrict__ zx, int ldz, __nv_bfloat16* __restrict__ planes, int parts,
+                  const int32_t* __restrict__ env_idx) {
   pdl_enter();
   const int b = blockIdx.y, g = blockIdx.z;
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= ldz) return;
+  const int e = kEnvs ? __ldg(&env_idx[b]) : b;
   const size_t row = (size_t)g * gridDim.y + b;
   float v = 0.f;
   if (k < nI) {
     const int2 rc = __ldg(&inner_rc[k]);
     const float* __restrict__ map = grp.win[g];
-    v = __ldg(&map[(size_t)b * env_stride + (size_t)(rc.x - grp.sy[g]) * pitch + (rc.y - grp.sx[g])]);
+    v = __ldg(&map[(size_t)e * env_stride + (size_t)(rc.x - grp.sy[g]) * pitch + (rc.y - grp.sx[g])]);
   } else if (k < nI + nO) {
     const int j = k - nI;
     if (xi != nullptr) {
@@ -46,7 +51,7 @@ atm_gather_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t
     } else {
       const unsigned long long stream_id = grp.stream_id[g];
       Philox rng(grp.seed[g]);
-      const uint4 r = rng((uint32_t)j, (uint32_t)b, (uint32_t)stream_id, (uint32_t)(stream_id >> 32));
+      const uint4 r = rng((uint32_t)j, (uint32_t)e, (uint32_t)stream_id, (uint32_t)(stream_id >> 32));
       v = box_muller(r.x, r.y).x;
     }
   }
@@ -99,21 +104,26 @@ __device__ __forceinline__ void block_reduce_ext(unsigned long long& lo, unsigne
 // add_row step 3 (OOPAO/Atmosphere.py:309): one CTA per environment writes the ring of the NEW window (ring index in
 // numpy boolean-mask order of `outerMask`, :263-264: row 0, then the (r,0),(r,M-1) pairs, then row M-1), reduces the
 // ring extrema and decides whether the tracked extrema survive.
+// kEnvs: CTA b writes environment env_idx[b] of nB (the extrema blocks hold nB environments); workspace rows stay b.
+template <bool kEnvs>
 __global__ void __launch_bounds__(256)
 atm_ring_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t env_stride,
-                const float* __restrict__ X, int ldx, int32_t* __restrict__ flag, int force_rescan) {
+                const float* __restrict__ X, int ldx, int32_t* __restrict__ flag, int force_rescan,
+                const int32_t* __restrict__ env_idx, int nB) {
   pdl_enter();
   const int b = blockIdx.x, g = blockIdx.y;
+  const int e = kEnvs ? __ldg(&env_idx[b]) : b;
+  const size_t nEnv = kEnvs ? (size_t)nB : (size_t)gridDim.x;
   const size_t row = (size_t)g * gridDim.x + b;
   const uint32_t win_offset = grp.win_offset[g];
   unsigned long long* __restrict__ ext = grp.ext[g];
-  float* __restrict__ w = grp.win[g] + (size_t)b * env_stride;
+  float* __restrict__ w = grp.win[g] + (size_t)e * env_stride;
   const float* __restrict__ xb = X + row * ldx;
   const int nO = 4 * M - 4;
   // Which lines became interior with this step: the window moved by (dy, dx) = new origin - previous origin (block 2 of
   // the extrema array remembers the previous one); origin - 1 along an axis exposes line 1 of that axis, + 1 line M - 2.
   // Unknown history (first call, forced rescan) -> all four edge lines of the interior.
-  unsigned long long* __restrict__ ext_prev = ext + 4 * (size_t)gridDim.x + 2 * b;
+  unsigned long long* __restrict__ ext_prev = ext + 4 * nEnv + 2 * e;
   const unsigned long long prev = *ext_prev;
   const int oy = win_offset / pitch, ox = win_offset % pitch;
   int line_r[2], line_c[2], nr = 0, nc = 0;                     // rows / columns of the window to merge
@@ -179,8 +189,8 @@ atm_ring_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t e
   __syncthreads();                       // the reduction scratch is reused
   block_reduce_ext(ilo, ihi);
   if (threadIdx.x == 0) {
-    unsigned long long* __restrict__ ext_in = ext + 2 * (size_t)gridDim.x;      // block 1: interior extrema
-    const unsigned long long old_lo = ext_in[2 * b], old_hi = ext_in[2 * b + 1];
+    unsigned long long* __restrict__ ext_in = ext + 2 * nEnv;                   // block 1: interior extrema
+    const unsigned long long old_lo = ext_in[2 * e], old_hi = ext_in[2 * e + 1];
     *ext_prev = (1ull << 32) | win_offset;
     auto retained = [&](unsigned long long pk) {
       const uint32_t pos = (uint32_t)pk;
@@ -192,10 +202,10 @@ atm_ring_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t e
       ilo = old_lo < ilo ? old_lo : ilo;
       ihi = old_hi > ihi ? old_hi : ihi;
     }
-    ext_in[2 * b] = ilo;                  // not ok: the edge lines only, the rescan merges the rest
-    ext_in[2 * b + 1] = ihi;
-    ext[2 * b] = ilo < lo ? ilo : lo;
-    ext[2 * b + 1] = ihi > hi ? ihi : hi;
+    ext_in[2 * e] = ilo;                  // not ok: the edge lines only, the rescan merges the rest
+    ext_in[2 * e + 1] = ihi;
+    ext[2 * e] = ilo < lo ? ilo : lo;
+    ext[2 * e + 1] = ihi > hi ? ihi : hi;
     flag[row] = ok ? 0 : 1;
   }
 }
@@ -205,15 +215,18 @@ atm_ring_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t e
 // running extrema are kept as (value, position) pairs under plain float comparisons and packed once at the end.  Rows
 // start on arbitrary columns (the window origin moves pixel by pixel), so the first / last vector of a row is masked.
 // Needs pitch and env_stride to be multiples of 4 floats (then every row has the same misalignment).
+template <bool kEnvs>
 __global__ void __launch_bounds__(256)
 atm_rescan_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t env_stride,
-                  const int32_t* __restrict__ flag, int rows_per_block) {
+                  const int32_t* __restrict__ flag, int rows_per_block, const int32_t* __restrict__ env_idx, int nB) {
   pdl_enter();
   const int b = blockIdx.y, g = blockIdx.z;
   if (__ldg(&flag[(size_t)g * gridDim.y + b]) == 0) return;
+  const int e = kEnvs ? __ldg(&env_idx[b]) : b;
+  const size_t nEnv = kEnvs ? (size_t)nB : (size_t)gridDim.y;
   const uint32_t win_offset = grp.win_offset[g];
   unsigned long long* __restrict__ ext = grp.ext[g];
-  const float* __restrict__ w = grp.win[g] + (size_t)b * env_stride;
+  const float* __restrict__ w = grp.win[g] + (size_t)e * env_stride;
   const int r_begin = 1 + blockIdx.x * rows_per_block;
   const int r_end = min(M - 1, r_begin + rows_per_block);
   const int mis = (int)((reinterpret_cast<uintptr_t>(w) >> 2) & 3);      // window column 0 sits `mis` floats into a 16-byte line
@@ -249,11 +262,11 @@ atm_rescan_kernel(const __grid_constant__ AtmGroup grp, int M, int pitch, size_t
   unsigned long long hi = vhi > -INFINITY ? pack(vhi, win_offset + phi) : 0ull;
   block_reduce_ext(lo, hi);
   if (threadIdx.x == 0 && r_begin < r_end) {
-    unsigned long long* __restrict__ ext_in = ext + 2 * (size_t)gridDim.y;       // block 1: interior extrema
-    atomicMin(&ext_in[2 * b], lo);
-    atomicMax(&ext_in[2 * b + 1], hi);
-    atomicMin(&ext[2 * b], lo);
-    atomicMax(&ext[2 * b + 1], hi);
+    unsigned long long* __restrict__ ext_in = ext + 2 * nEnv;                    // block 1: interior extrema
+    atomicMin(&ext_in[2 * e], lo);
+    atomicMax(&ext_in[2 * e + 1], hi);
+    atomicMin(&ext[2 * e], lo);
+    atomicMax(&ext[2 * e + 1], hi);
   }
 }
 
@@ -347,12 +360,15 @@ __device__ __forceinline__ void phase_rows(const float* __restrict__ tbase, floa
   }
 }
 
+// kEnvs: grid layer z computes environment env_idx[z] (same arithmetic as the whole-batch launch, per environment)
+template <bool kEnvs>
 __global__ void __launch_bounds__(kPhThreadsX * kPhThreadsY)
-atm_phase_kernel(const __grid_constant__ AtmPhaseParams p, int R, float opd_scale, float* __restrict__ opd_out) {
+atm_phase_kernel(const __grid_constant__ AtmPhaseParams p, int R, float opd_scale, float* __restrict__ opd_out,
+                 const int32_t* __restrict__ env_idx) {
   pdl_enter();
   __shared__ __align__(128) float tile[2][kPhBufFloats];
   __shared__ __align__(8) uint64_t bar[2];
-  const int b = blockIdx.z;
+  const int b = kEnvs ? __ldg(&env_idx[blockIdx.z]) : (int)blockIdx.z;
   const int j0 = blockIdx.x * kPhTileW, i0 = blockIdx.y * kPhTileH;
   const int tx = threadIdx.x, ty = threadIdx.y;
   const bool leader = (tx == 0 && ty == 0);
@@ -431,12 +447,11 @@ static int rows_per_block_for(int B, int M) {
   return (M + chunks - 1) / chunks;
 }
 
-extern "C" {
+namespace {
 
-int aoenv_atm_gather_multi(const void* const* wins, const int32_t* sx, const int32_t* sy, const uint64_t* seeds,
-                           const uint64_t* stream_ids, int G, int B, int M, int pitch, int64_t env_stride,
-                           const int32_t* inner_rc, int nI, int nO, const float* xi, float* zx, int ldz, void* zx_planes,
-                           int parts, void* stream) {
+int gather_launch(const void* const* wins, const int32_t* sx, const int32_t* sy, const uint64_t* seeds, const uint64_t* stream_ids,
+                  int G, int B, int M, int pitch, int64_t env_stride, const int32_t* inner_rc, int nI, int nO, const float* xi,
+                  float* zx, int ldz, void* zx_planes, int parts, const int32_t* env_idx, void* stream) {
   AOENV_CHECK_ARG(G > 0 && G <= AOENV_MAX_LAYERS, "atm_gather: %d layers in one group (max %d)", G, AOENV_MAX_LAYERS);
   AOENV_CHECK_ARG(B > 0 && B <= 65535 && M > 6 && pitch >= M && env_stride >= (int64_t)M * pitch, "atm_gather: bad shape B=%d M=%d pitch=%d", B, M, pitch);
   AOENV_CHECK_ARG(ldz >= nI + nO, "atm_gather: ldz=%d < nI+nO=%d", ldz, nI + nO);
@@ -452,10 +467,69 @@ int aoenv_atm_gather_multi(const void* const* wins, const int32_t* sx, const int
     grp.stream_id[g] = stream_ids ? stream_ids[g] : 0;
   }
   dim3 grid((ldz + 255) / 256, B, G);
-  AOENV_LAUNCH(atm_gather_kernel, grid, 256, 0, (cudaStream_t)stream, grp, M, pitch, (size_t)env_stride, (const int2*)inner_rc, nI, nO,
-                                                            xi, zx, ldz, (__nv_bfloat16*)zx_planes, parts);
+  if (env_idx)
+    AOENV_LAUNCH(atm_gather_kernel<true>, grid, 256, 0, (cudaStream_t)stream, grp, M, pitch, (size_t)env_stride,
+                 (const int2*)inner_rc, nI, nO, xi, zx, ldz, (__nv_bfloat16*)zx_planes, parts, env_idx);
+  else
+    AOENV_LAUNCH(atm_gather_kernel<false>, grid, 256, 0, (cudaStream_t)stream, grp, M, pitch, (size_t)env_stride,
+                 (const int2*)inner_rc, nI, nO, xi, zx, ldz, (__nv_bfloat16*)zx_planes, parts, env_idx);
   AOENV_LAUNCH_CHECK("atm_gather");
   return 0;
+}
+
+// rows = workspace rows per layer (B, or k listed environments); nB = environments in the extrema blocks
+int ring_launch(void* const* wins, const int64_t* win_offsets, void* const* exts, int G, int rows, int nB, int M, int pitch,
+                int64_t env_stride, int nO, const float* X, int ldx, int32_t* flag, int force_rescan, const int32_t* env_idx,
+                void* stream) {
+  AOENV_CHECK_ARG(G > 0 && G <= AOENV_MAX_LAYERS, "atm_ring: %d layers in one group (max %d)", G, AOENV_MAX_LAYERS);
+  AOENV_CHECK_ARG(rows > 0 && rows <= 65535 && nB >= rows && M > 6 && pitch >= M && pitch % 4 == 0 && env_stride % 4 == 0,
+                  "atm_ring: bad shape (pitch and env_stride must be multiples of 4 floats)");
+  AOENV_CHECK_ARG(nO == 4 * M - 4 && ldx >= nO, "atm_ring: ring has %d pixels, got nO=%d ldx=%d", 4 * M - 4, nO, ldx);
+  AtmGroup grp{};
+  for (int g = 0; g < G; ++g) {
+    AOENV_CHECK_ARG(win_offsets[g] >= 0 && win_offsets[g] + (int64_t)M * pitch <= env_stride + pitch && env_stride < (1ll << 32),
+                    "atm_ring: window leaves the canvas");
+    grp.win[g] = (float*)wins[g];
+    grp.ext[g] = (unsigned long long*)exts[g];
+    grp.win_offset[g] = (uint32_t)win_offsets[g];
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  if (env_idx)
+    AOENV_LAUNCH(atm_ring_kernel<true>, dim3(rows, G), 256, 0, s, grp, M, pitch, (size_t)env_stride, X, ldx, flag, force_rescan,
+                 env_idx, nB);
+  else
+    AOENV_LAUNCH(atm_ring_kernel<false>, dim3(rows, G), 256, 0, s, grp, M, pitch, (size_t)env_stride, X, ldx, flag, force_rescan,
+                 env_idx, nB);
+  AOENV_LAUNCH_CHECK("atm_ring");
+  const int rpb = 32;                          // >= 8 CTAs per flagged environment; unflagged ones exit at once (8 rows per CTA measured slower: 169 vs 138 us)
+  dim3 grid((M - 2 + rpb - 1) / rpb, rows, G);
+  if (env_idx)
+    AOENV_LAUNCH(atm_rescan_kernel<true>, grid, 256, 0, s, grp, M, pitch, (size_t)env_stride, flag, rpb, env_idx, nB);
+  else
+    AOENV_LAUNCH(atm_rescan_kernel<false>, grid, 256, 0, s, grp, M, pitch, (size_t)env_stride, flag, rpb, env_idx, nB);
+  AOENV_LAUNCH_CHECK("atm_rescan");
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int aoenv_atm_gather_multi(const void* const* wins, const int32_t* sx, const int32_t* sy, const uint64_t* seeds,
+                           const uint64_t* stream_ids, int G, int B, int M, int pitch, int64_t env_stride,
+                           const int32_t* inner_rc, int nI, int nO, const float* xi, float* zx, int ldz, void* zx_planes,
+                           int parts, void* stream) {
+  return gather_launch(wins, sx, sy, seeds, stream_ids, G, B, M, pitch, env_stride, inner_rc, nI, nO, xi, zx, ldz, zx_planes,
+                       parts, nullptr, stream);
+}
+
+int aoenv_atm_gather_envs(const void* const* wins, const uint64_t* seeds, const uint64_t* stream_ids, int G,
+                          const int32_t* env_idx, int k, int M, int pitch, int64_t env_stride, const int32_t* inner_rc, int nI,
+                          int nO, float* zx, int ldz, void* zx_planes, int parts, void* stream) {
+  AOENV_CHECK_ARG(env_idx != nullptr, "atm_gather_envs: no environment list");
+  const int32_t zero[AOENV_MAX_LAYERS] = {};
+  return gather_launch(wins, zero, zero, seeds, stream_ids, G, k, M, pitch, env_stride, inner_rc, nI, nO, nullptr, zx, ldz,
+                       zx_planes, parts, env_idx, stream);
 }
 
 int aoenv_atm_gather(const float* win, int B, int M, int pitch, int64_t env_stride, int sx, int sy,
@@ -470,26 +544,14 @@ int aoenv_atm_gather(const float* win, int B, int M, int pitch, int64_t env_stri
 
 int aoenv_atm_ring_multi(void* const* wins, const int64_t* win_offsets, void* const* exts, int G, int B, int M, int pitch,
                          int64_t env_stride, int nO, const float* X, int ldx, int32_t* flag, int force_rescan, void* stream) {
-  AOENV_CHECK_ARG(G > 0 && G <= AOENV_MAX_LAYERS, "atm_ring: %d layers in one group (max %d)", G, AOENV_MAX_LAYERS);
-  AOENV_CHECK_ARG(B > 0 && B <= 65535 && M > 6 && pitch >= M && pitch % 4 == 0 && env_stride % 4 == 0,
-                  "atm_ring: bad shape (pitch and env_stride must be multiples of 4 floats)");
-  AOENV_CHECK_ARG(nO == 4 * M - 4 && ldx >= nO, "atm_ring: ring has %d pixels, got nO=%d ldx=%d", 4 * M - 4, nO, ldx);
-  AtmGroup grp{};
-  for (int g = 0; g < G; ++g) {
-    AOENV_CHECK_ARG(win_offsets[g] >= 0 && win_offsets[g] + (int64_t)M * pitch <= env_stride + pitch && env_stride < (1ll << 32),
-                    "atm_ring: window leaves the canvas");
-    grp.win[g] = (float*)wins[g];
-    grp.ext[g] = (unsigned long long*)exts[g];
-    grp.win_offset[g] = (uint32_t)win_offsets[g];
-  }
-  cudaStream_t s = (cudaStream_t)stream;
-  AOENV_LAUNCH(atm_ring_kernel, dim3(B, G), 256, 0, s, grp, M, pitch, (size_t)env_stride, X, ldx, flag, force_rescan);
-  AOENV_LAUNCH_CHECK("atm_ring");
-  const int rpb = 32;                          // >= 8 CTAs per flagged environment; unflagged ones exit at once (8 rows per CTA measured slower: 169 vs 138 us)
-  dim3 grid((M - 2 + rpb - 1) / rpb, B, G);
-  AOENV_LAUNCH(atm_rescan_kernel, grid, 256, 0, s, grp, M, pitch, (size_t)env_stride, flag, rpb);
-  AOENV_LAUNCH_CHECK("atm_rescan");
-  return 0;
+  return ring_launch(wins, win_offsets, exts, G, B, B, M, pitch, env_stride, nO, X, ldx, flag, force_rescan, nullptr, stream);
+}
+
+int aoenv_atm_ring_envs(void* const* wins, const int64_t* win_offsets, void* const* exts, int G, const int32_t* env_idx, int k,
+                        int B, int M, int pitch, int64_t env_stride, int nO, const float* X, int ldx, int32_t* flag,
+                        void* stream) {
+  AOENV_CHECK_ARG(env_idx != nullptr, "atm_ring_envs: no environment list");
+  return ring_launch(wins, win_offsets, exts, G, k, B, M, pitch, env_stride, nO, X, ldx, flag, 1, env_idx, stream);
 }
 
 int aoenv_atm_ring(float* win, int B, int M, int pitch, int64_t env_stride, int64_t win_offset, int nO, const float* X,
@@ -512,10 +574,16 @@ int aoenv_atm_compact(const float* src_win, float* dst_win, int B, int M, int pi
   return 0;
 }
 
-int aoenv_atm_phase(const float* const* h_canvas, const uint64_t* const* h_ext, const int32_t* h_org, int nLayer, int B,
-                    int R, int M, int Mc, int pitch, int fp_off, const int32_t* h_row_off, const int32_t* h_col_off,
-                    const float* h_wrow, const float* h_wcol, const float* h_weight, float opd_scale, float* opd_out,
-                    void* stream) {
+}  // extern "C"
+
+namespace {
+
+// grid layers: B environments, or the k of env_idx (the tensor maps always describe the whole batch of B canvases)
+int phase_launch(const float* const* h_canvas, const uint64_t* const* h_ext, const int32_t* h_org, int nLayer, int B, int R,
+                 int M, int Mc, int pitch, int fp_off, const int32_t* h_row_off, const int32_t* h_col_off, const float* h_wrow,
+                 const float* h_wcol, const float* h_weight, float opd_scale, const int32_t* env_idx, int k, float* opd_out,
+                 void* stream) {
+  AOENV_CHECK_ARG(k > 0 && k <= B, "atm_phase: %d environments listed of %d", k, B);
   AOENV_CHECK_ARG(nLayer >= 1 && nLayer <= AOENV_MAX_LAYERS, "atm_phase: nLayer=%d out of range", nLayer);
   AOENV_CHECK_ARG(B > 0 && B <= 65535, "atm_phase: B=%d out of range (1..65535)", B);
   AOENV_CHECK_ARG(pitch % 4 == 0 && pitch >= Mc && Mc >= M, "atm_phase: bad canvas Mc=%d pitch=%d", Mc, pitch);
@@ -555,10 +623,34 @@ int aoenv_atm_phase(const float* const* h_canvas, const uint64_t* const* h_ext, 
     p.weight[l] = h_weight[l];
   }
   dim3 block(kPhThreadsX, kPhThreadsY);
-  dim3 grid((R + kPhTileW - 1) / kPhTileW, (R + kPhTileH - 1) / kPhTileH, B);
-  AOENV_LAUNCH(atm_phase_kernel, grid, block, 0, (cudaStream_t)stream, p, R, opd_scale, opd_out);
+  dim3 grid((R + kPhTileW - 1) / kPhTileW, (R + kPhTileH - 1) / kPhTileH, k);
+  if (env_idx)
+    AOENV_LAUNCH(atm_phase_kernel<true>, grid, block, 0, (cudaStream_t)stream, p, R, opd_scale, opd_out, env_idx);
+  else
+    AOENV_LAUNCH(atm_phase_kernel<false>, grid, block, 0, (cudaStream_t)stream, p, R, opd_scale, opd_out, env_idx);
   AOENV_LAUNCH_CHECK("atm_phase");
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int aoenv_atm_phase(const float* const* h_canvas, const uint64_t* const* h_ext, const int32_t* h_org, int nLayer, int B,
+                    int R, int M, int Mc, int pitch, int fp_off, const int32_t* h_row_off, const int32_t* h_col_off,
+                    const float* h_wrow, const float* h_wcol, const float* h_weight, float opd_scale, float* opd_out,
+                    void* stream) {
+  return phase_launch(h_canvas, h_ext, h_org, nLayer, B, R, M, Mc, pitch, fp_off, h_row_off, h_col_off, h_wrow, h_wcol, h_weight,
+                      opd_scale, nullptr, B, opd_out, stream);
+}
+
+int aoenv_atm_phase_envs(const float* const* h_canvas, const uint64_t* const* h_ext, const int32_t* h_org, int nLayer, int B,
+                         int R, int M, int Mc, int pitch, int fp_off, const int32_t* h_row_off, const int32_t* h_col_off,
+                         const float* h_wrow, const float* h_wcol, const float* h_weight, float opd_scale, const int32_t* env_idx,
+                         int k, float* opd_out, void* stream) {
+  AOENV_CHECK_ARG(env_idx != nullptr, "atm_phase_envs: no environment list");
+  return phase_launch(h_canvas, h_ext, h_org, nLayer, B, R, M, Mc, pitch, fp_off, h_row_off, h_col_off, h_wrow, h_wcol, h_weight,
+                      opd_scale, env_idx, k, opd_out, stream);
 }
 
 }  // extern "C"

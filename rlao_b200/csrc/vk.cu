@@ -26,10 +26,16 @@ __device__ __forceinline__ float2 vk_normals(const Philox& rng, const float* __r
   return box_muller(w.x, w.y);
 }
 
+// Philox stream of screen s: screen0 + s, or screen0 + env_idx[s] when the screens go to a list of environments
+__device__ __forceinline__ uint32_t vk_stream(uint32_t screen0, const int32_t* __restrict__ env_idx, int s) {
+  return screen0 + (uint32_t)(env_idx ? __ldg(&env_idx[s]) : s);
+}
+
 // planes[(s, b)][k]: k < N -> Re cn'[a = k][b], N <= k < 2N -> Im cn'[a = k - N][b], zero beyond (operand of pass A)
 __global__ void __launch_bounds__(256)
 vk_spectrum_kernel(unsigned long long seed, uint32_t screen0, int S, int N, const float* __restrict__ amp,
-                   const float* __restrict__ inject, __nv_bfloat16* __restrict__ planes, int Kp, int parts) {
+                   const float* __restrict__ inject, __nv_bfloat16* __restrict__ planes, int Kp, int parts,
+                   const int32_t* __restrict__ env_idx) {
   const int s = blockIdx.z, b = blockIdx.y;
   const int a = blockIdx.x * blockDim.x + threadIdx.x;
   if (a >= Kp) return;
@@ -38,7 +44,7 @@ vk_spectrum_kernel(unsigned long long seed, uint32_t screen0, int S, int N, cons
   if (a < N) {
     Philox rng(seed);
     const uint32_t flat = (uint32_t)a * N + b;
-    const float2 z = vk_normals(rng, inject, S, N, inject ? (uint32_t)s : screen0 + s, flat);
+    const float2 z = vk_normals(rng, inject, S, N, inject ? (uint32_t)s : vk_stream(screen0, env_idx, s), flat);
     const float w = __ldg(&amp[flat]);                       // sqrt(PSD) del_f (-1)^(a+b)
     store_bf16_planes(planes, stride, row * Kp + a, parts, z.x * w);
     store_bf16_planes(planes, stride, row * Kp + N + a, parts, z.y * w);
@@ -83,11 +89,12 @@ struct VkSubharmonics {
   float2 mx[3][2], my[3][2];   // means of ex / ey over the grid (for the analytic mean of the low-frequency screen)
 };
 
-// screen = hi + lo - mean(lo), stored into the interior of the layer window (the reference's layer.phase)
+// screen = hi + lo - mean(lo), stored into the interior of the layer window (the reference's layer.phase) of environment
+// s, or env_idx[s]
 __global__ void __launch_bounds__(256)
 vk_finish_kernel(const float* __restrict__ hi, int ldh, unsigned long long seed, uint32_t screen0, int S, int N,
                  const float* __restrict__ inject, const __grid_constant__ VkSubharmonics sh, float* __restrict__ dst, int pitch,
-                 size_t env_stride) {
+                 size_t env_stride, const int32_t* __restrict__ env_idx) {
   __shared__ float2 cs[3][2][2];
   __shared__ float mean;
   const int s = blockIdx.z, y = blockIdx.y;
@@ -96,7 +103,7 @@ vk_finish_kernel(const float* __restrict__ hi, int ldh, unsigned long long seed,
     // parts, the stream positions 18 (p-1) + 3 i + j of the real-part draw, and 9 further on for its imaginary parts.
     const int p = threadIdx.x / 4, i = (threadIdx.x >> 1) & 1, j = threadIdx.x & 1;
     Philox rng(seed);
-    const uint32_t sid = inject ? (uint32_t)s : screen0 + s;
+    const uint32_t sid = inject ? (uint32_t)s : vk_stream(screen0, env_idx, s);
     const float re = vk_normals(rng, inject, S, N, sid, 18u * p + 3u * i + j).x;
     const float im = vk_normals(rng, inject, S, N, sid, 18u * p + 9u + 3u * i + j).x;
     cs[p][i][j] = make_float2(re * sh.amp[p][i][j], im * sh.amp[p][i][j]);
@@ -129,7 +136,7 @@ vk_finish_kernel(const float* __restrict__ hi, int ldh, unsigned long long seed,
       }
       t[p][j] = acc;
     }
-  float* __restrict__ out = dst + (size_t)s * env_stride + (size_t)y * pitch;
+  float* __restrict__ out = dst + (size_t)(env_idx ? __ldg(&env_idx[s]) : s) * env_stride + (size_t)y * pitch;
   const float* __restrict__ h = hi + ((size_t)s * N + y) * ldh;
   for (int x = threadIdx.x; x < N; x += blockDim.x) {
     float lo = 0.f;
@@ -148,19 +155,19 @@ vk_finish_kernel(const float* __restrict__ hi, int ldh, unsigned long long seed,
 
 using namespace aoenv;
 
-extern "C" {
+namespace {
 
-int aoenv_vk_screens(uint64_t seed, uint32_t screen0, int S, int N, const float* amp, const float* inject, const void* wa_planes,
-                     const void* wb_planes, int Kp, int parts, const float* sh_ex, const float* sh_ey, const float* h_amp,
-                     const float* h_mx, const float* h_my, void* work_planes, float* work_a, int lda, float* work_b, int ldb,
-                     float* dst, int pitch, int64_t env_stride, void* stream) {
+int vk_screens(uint64_t seed, uint32_t screen0, const int32_t* env_idx, int S, int N, const float* amp, const float* inject,
+               const void* wa_planes, const void* wb_planes, int Kp, int parts, const float* sh_ex, const float* sh_ey,
+               const float* h_amp, const float* h_mx, const float* h_my, void* work_planes, float* work_a, int lda, float* work_b,
+               int ldb, float* dst, int pitch, int64_t env_stride, void* stream) {
   AOENV_CHECK_ARG(S > 0 && 2 * S <= 65535 && N >= 8 && N <= 32768, "vk_screens: bad shape S=%d N=%d", S, N);
   AOENV_CHECK_ARG(Kp >= 2 * N && Kp % 16 == 0 && lda >= 2 * N && ldb >= N && pitch >= N, "vk_screens: bad leading dimensions");
   AOENV_CHECK_ARG(parts == 2 || parts == 3, "vk_screens: parts must be 2 or 3");
   cudaStream_t st = (cudaStream_t)stream;
   __nv_bfloat16* planes = (__nv_bfloat16*)work_planes;
   // random spectrum, operand form of pass A
-  vk_spectrum_kernel<<<dim3((Kp + 255) / 256, N, S), 256, 0, st>>>(seed, screen0, S, N, amp, inject, planes, Kp, parts);
+  vk_spectrum_kernel<<<dim3((Kp + 255) / 256, N, S), 256, 0, st>>>(seed, screen0, S, N, amp, inject, planes, Kp, parts, env_idx);
   AOENV_LAUNCH_CHECK("vk_spectrum");
   // pass A: U[(s, b)][(y, re|im)] = sum_(a, re|im) cn'[(s, b)][(a, re|im)] WA[(y, re|im)][(a, re|im)]
   int rc = aoenv_gemm_tn_tc(planes, wa_planes, Kp, parts, work_a, lda, S * N, 2 * N, Kp, 1.0f, stream);
@@ -179,9 +186,31 @@ int aoenv_vk_screens(uint64_t seed, uint32_t screen0, int S, int N, const float*
       sh.mx[p][i] = make_float2(h_mx[(p * 2 + i) * 2], h_mx[(p * 2 + i) * 2 + 1]);
       sh.my[p][i] = make_float2(h_my[(p * 2 + i) * 2], h_my[(p * 2 + i) * 2 + 1]);
     }
-  vk_finish_kernel<<<dim3(1, N, S), 256, 0, st>>>(work_b, ldb, seed, screen0, S, N, inject, sh, dst, pitch, (size_t)env_stride);
+  vk_finish_kernel<<<dim3(1, N, S), 256, 0, st>>>(work_b, ldb, seed, screen0, S, N, inject, sh, dst, pitch, (size_t)env_stride,
+                                              env_idx);
   AOENV_LAUNCH_CHECK("vk_finish");
   return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int aoenv_vk_screens(uint64_t seed, uint32_t screen0, int S, int N, const float* amp, const float* inject, const void* wa_planes,
+                     const void* wb_planes, int Kp, int parts, const float* sh_ex, const float* sh_ey, const float* h_amp,
+                     const float* h_mx, const float* h_my, void* work_planes, float* work_a, int lda, float* work_b, int ldb,
+                     float* dst, int pitch, int64_t env_stride, void* stream) {
+  return vk_screens(seed, screen0, nullptr, S, N, amp, inject, wa_planes, wb_planes, Kp, parts, sh_ex, sh_ey, h_amp, h_mx, h_my,
+                    work_planes, work_a, lda, work_b, ldb, dst, pitch, env_stride, stream);
+}
+
+int aoenv_vk_screens_envs(uint64_t seed, uint32_t screen0, const int32_t* env_idx, int S, int N, const float* amp,
+                          const void* wa_planes, const void* wb_planes, int Kp, int parts, const float* sh_ex, const float* sh_ey,
+                          const float* h_amp, const float* h_mx, const float* h_my, void* work_planes, float* work_a, int lda,
+                          float* work_b, int ldb, float* dst, int pitch, int64_t env_stride, void* stream) {
+  AOENV_CHECK_ARG(env_idx != nullptr, "vk_screens_envs: no environment list");
+  return vk_screens(seed, screen0, env_idx, S, N, amp, nullptr, wa_planes, wb_planes, Kp, parts, sh_ex, sh_ey, h_amp, h_mx, h_my,
+                    work_planes, work_a, lda, work_b, ldb, dst, pitch, env_stride, stream);
 }
 
 }  // extern "C"

@@ -184,8 +184,10 @@ class ScreenSynth:
         self.h_amp = np.ascontiguousarray(amp_lo, dtype=np.float32)
         self.h_mean = np.ascontiguousarray(pack(ex.mean(axis=2)), dtype=np.float32)
 
-    def generate(self, seed, screen0, S, dst_ptr, pitch, env_stride, inject=None):
-        """Writes S screens into the windows starting at device address dst_ptr (row 1 / column 1 of environment 0)."""
+    def generate(self, seed, screen0, S, dst_ptr, pitch, env_stride, inject=None, env_idx=None):
+        """Writes S screens into the windows starting at device address dst_ptr (row 1 / column 1 of environment 0); with
+        env_idx (int32 device tensor of S environments), screen s goes to environment env_idx[s] from its stream
+        screen0 + env_idx[s] (aoenv_vk_screens_envs)."""
         import ctypes as C
         from .. import _lib
         lib, N, Kp, dev = _lib.load(), self.N, self.Kp, self.device
@@ -198,6 +200,13 @@ class ScreenSynth:
         f = lambda a: a.ctypes.data_as(C.c_void_p)
         for s0 in range(0, S, chunk):
             m = min(chunk, S - s0)
+            if env_idx is not None:
+                _lib.check(lib.aoenv_vk_screens_envs(
+                    C.c_uint64(seed & 0xFFFFFFFFFFFFFFFF), C.c_uint32(screen0 & 0xFFFFFFFF), _lib.ptr(env_idx[s0:s0 + m]), m, N,
+                    _lib.ptr(self.amp), _lib.ptr(self.WA.planes()), _lib.ptr(self.WB.planes()), Kp, self.parts,
+                    _lib.ptr(self.sh_ex), _lib.ptr(self.sh_ex), f(self.h_amp), f(self.h_mean), f(self.h_mean), _lib.ptr(planes),
+                    _lib.ptr(wa), lda, _lib.ptr(wb), ldb, dst_ptr, pitch, env_stride, _lib.stream_ptr(dev)), "vk_screens_envs")
+                continue
             inj = None
             if inject is not None:
                 inj = torch.as_tensor(inject[s0:s0 + m], dtype=torch.float32, device=dev).contiguous()
