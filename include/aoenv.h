@@ -254,7 +254,8 @@ int aoenv_detector_integrate(float* frame, int B, int rows, int cols, const aoen
 /* The camera of the WFS as its own step: the same chain applied in place to B noise-free frames of nS x nS lenslets of
  * n x n pixels, and envmax [B] (or [1] when shared_max) = maximum over the pixels of the valid lenslets AFTER the
  * camera (the centroiding threshold of ShackHartmann.py:314-316 is taken on the detector output).  This is the second
- * half of aoenv_shwfs_frame with a detector; aoenv_shwfs_fused + this + aoenv_shwfs_slopes is the noisy step. */
+ * half of aoenv_shwfs_frame with a detector; aoenv_shwfs_fused + this + aoenv_shwfs_slopes is the noisy step.  Any n > 0
+ * (the camera works per pixel and looks up the lenslet of a pixel only for the maximum). */
 int aoenv_shwfs_camera(float* frame, const uint8_t* valid, int B, int nS, int n, const aoenv_detector_t* det, int shared_max,
                        int32_t* envmax, void* stream);
 
@@ -274,7 +275,8 @@ int aoenv_set_wfs6_variant(int variant);
  * stats [B][4] (float64): sums over pupil pixels of {a, a^2, t, t^2}, a = opd_a - opd_a[centre], t = opd - opd[centre]
  * in metres (centred on the pupil-centre pixel: only variances are derived from them), for env.total /
  * env.residual / get_strehl (MAIN/OOPAOEnv/OOPAOEnvRazor.py:484,502,604-605). May be NULL.
- * n (pixels per lenslet) must be one of the compiled sizes (4, 6, 8). */
+ * n (pixels per lenslet) must be one of the compiled sizes (4, 6, 8, 10, 12).  n = 10, 12 run on n / 2 lanes per lenslet
+ * and only with the default frame variant (aoenv_set_wfs6_variant(0)); another variant is rejected for them. */
 int aoenv_shwfs_frame(const float* opd_a, const float* opd_b, const float* pupil, const float* amp,
                       const uint8_t* valid, int B, int nS, int n, float phase_scale,
                       const aoenv_detector_t* det, int shared_max,
@@ -284,7 +286,8 @@ int aoenv_shwfs_frame(const float* opd_a, const float* opd_b, const float* pupil
  * lenslet map's axis 1 -> X and axis 2 -> Y, NaN/Inf -> 0, minus reference, divided by slopes_units.
  * valid_idx [nV]: lenslet numbers k = i*nS + j of the valid lenslets (row-major); ref_xy [2][nV].
  * slopes [B][lds]: first nV entries X, next nV entries Y (= wfs.signal).  slope_planes (nullable): [parts][B][lds]
- * bf16, the same vector as operand planes of aoenv_gemm_tn_tc (the reconstruction), written in the same pass. */
+ * bf16, the same vector as operand planes of aoenv_gemm_tn_tc (the reconstruction), written in the same pass.
+ * n: 4, 6, 8, 10 or 12. */
 int aoenv_shwfs_slopes(const float* frame, const int32_t* envmax, int shared_max, const int32_t* valid_idx,
                        int nV, const float* ref_xy, float inv_units, float threshold_cog, int B, int nS, int n,
                        float* slopes, int lds, void* slope_planes, int parts, void* stream);
@@ -304,7 +307,8 @@ int aoenv_shwfs_slopes(const float* frame, const int32_t* envmax, int shared_max
  *   if invalid.  groups: warp groups per CTA.
  *   slopes (nullable; then only the frame is produced, envmax is reset for the camera pass) / slope_planes / ref_xy /
  *   inv_units / threshold_cog / envmax / stats: as in aoenv_shwfs_slopes and aoenv_shwfs_frame, except that stats
- *   holds the plain sums {sum a, sum a^2, sum t, sum t^2} over the pupil (a = opd_a, t = opd_a + DM). */
+ *   holds the plain sums {sum a, sum a^2, sum t, sum t^2} over the pupil (a = opd_a, t = opd_a + DM).
+ *   n: 4, 6, 8 only (other sizes are rejected). */
 typedef struct {
   const float* rows;             /* [B][nActP][R] T = C gx from aoenv_dm_rows (rows >= nAct are zero); NULL = no separable DM */
   const float* wlr;              /* [R][2 * pad4((WL+1)/2)] weights of pixel row y on the actuator rows ilr[y / n] + t, t < WL,  */
@@ -328,7 +332,8 @@ int aoenv_shwfs_fused(const float* opd_a, const float* opd_b, const aoenv_dm_sep
  * atmosphere's centre value — the variance is shift invariant).
  * order (nullable) [nS*nS]: a permutation of the lenslet numbers, the valid (lit) ones first: thread k works on lenslet
  * order[k], so whole warps are lit or dark and the dark ones skip the transform (21 % of the lenslets of a circular pupil).
- * The variants selected by aoenv_set_wfs6_variant ignore `dm` = NULL-only and `order`. */
+ * The variants selected by aoenv_set_wfs6_variant ignore `dm` = NULL-only and `order`.  n: as aoenv_shwfs_frame (4, 6, 8, 10,
+ * 12); WL 14 or 18 for every n (the window is counted in actuator rows, and a lenslet spans about one actuator pitch). */
 int aoenv_shwfs_frame_dm(const float* opd_a, const float* opd_b, const aoenv_dm_sep_t* dm, const int32_t* order,
                          const float* pupil, const float* amp, const uint8_t* valid, int B, int nS, int n, float phase_scale,
                          const aoenv_detector_t* det, int shared_max, float* frame, int32_t* envmax, double* stats,
@@ -377,7 +382,7 @@ int aoenv_sh_step(const aoenv_sh_step_t* c, int parts, const float* opd_a, const
  * reference slopes / slope units (ShackHartmann.py:254-312) and the interaction matrix pushes
  * (calibration/InteractionMatrix.py:79-84), whose 1 nm pokes move the spots by ~1e-3 pixel.  opd [F][R][R]
  * float32 (OPD_no_pupil, metres); frame [F][R][R], slopes [F][lds], ref_xy [2][nV] float64; envmax [F] (or [1]
- * when shared_max) scratch.  */
+ * when shared_max) scratch.  n: 4, 6, 8, 10 or 12. */
 int aoenv_shwfs_measure_f64(const float* opd, const float* pupil, const float* amp, const uint8_t* valid,
                             const int32_t* valid_idx, int nV, const double* ref_xy, double inv_units, double threshold_cog,
                             int F, int nS, int n, double phase_scale, int shared_max, double* frame, uint64_t* envmax,
@@ -397,14 +402,15 @@ int aoenv_shwfs_measure_f64(const float* opd, const float* pupil, const float* a
  *   float64 with the definition of aoenv_shwfs_frame_dm (with `dm`, the total is centred on the atmosphere's centre value).
  * One CTA per (environment, strip of lenslet rows): the strip's pixel rows and a one-row halo are staged in shared memory with
  * 128-bit loads (64-bit when R % 4 != 0), the DM surface is evaluated in registers and never written; slopes are reduced
- * without atomics (deterministic).  Two launches when stats is given (its reset, then the kernel), else one. */
+ * without atomics (deterministic).  Two launches when stats is given (its reset, then the kernel), else one.
+ * n: 4, 6, 8, 10 or 12; with `dm`, WL 14 or 18. */
 int aoenv_shwfs_geometric(const float* opd_a, const float* opd_b, const aoenv_dm_sep_t* dm, const float* pupil,
                           const float* flux, const int32_t* valid_idx, int nV, int B, int nS, int n, float phase_scale,
                           float inv_units, float* slopes, int lds, void* slope_planes, int parts, double* stats, void* stream);
 
 /* Calibration-grade twin (init only: slope units, interaction-matrix pushes): the same measurement in float64 arithmetic on
  * F wavefronts opd [F][R][R] (float32, OPD_no_pupil, metres); slopes [F][lds] float64 = gradient means * phase_scale *
- * inv_units. */
+ * inv_units.  n: 4, 6, 8, 10 or 12. */
 int aoenv_shwfs_geometric_f64(const float* opd, const float* flux, const int32_t* valid_idx, int nV, int F, int nS, int n,
                               double phase_scale, double inv_units, double* slopes, int lds, void* stream);
 

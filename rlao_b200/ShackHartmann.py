@@ -19,7 +19,8 @@ from . import _lib, gemm
 from .DeformableMirror import DMSurfaceRef
 from .Detector import Detector
 
-_SUPPORTED_N = (4, 6, 8)
+_SUPPORTED_N = (4, 6, 8, 10, 12)
+_FUSED_N = (4, 6, 8)              # the cluster-fused cross-check kernel (AOENV_WFS=fused) and the alternative frame variants
 
 
 class ShackHartmann:
@@ -204,6 +205,9 @@ class ShackHartmann:
         if plan is not None:
             return plan
         lib, nS, n, dev = _lib.load(), self.nSubap, self.n_pix_subap, self.device
+        if n not in _FUSED_N:
+            raise NotImplementedError(f"the fused WFS kernel (AOENV_WFS=fused) is compiled for {_FUSED_N} pixels per "
+                                      f"subaperture, not {n}")
         R = nS * n
         groups = int(os.environ.get("AOENV_WFS_GROUPS", "4"))
         valid = self.valid_subapertures

@@ -17,32 +17,6 @@ constexpr int kMaxN = 8;                 // pixels per lenslet side
 // phasor exp(-i pi (N+1)/N x) of ShackHartmann.py:208-209.
 __constant__ float2 c_tw[2 * kMaxN * kMaxN];
 __constant__ double2 c_twd[2 * kMaxN * kMaxN];   // float64 copy for the calibration-grade kernels
-static int g_tw_n[64] = {0};             // per device: n for which c_tw / c_twd are currently valid
-static std::mutex g_tw_mutex;
-
-static int ensure_twiddles(int n, cudaStream_t stream) {
-  int dev = 0;
-  cudaGetDevice(&dev);
-  std::lock_guard<std::mutex> lock(g_tw_mutex);
-  if (dev < 64 && g_tw_n[dev] == n) return 0;
-  const int N = 2 * n;
-  float2 h[2 * kMaxN * kMaxN];
-  double2 hd[2 * kMaxN * kMaxN];
-  for (int u = 0; u < N; ++u)
-    for (int a = 0; a < n; ++a) {
-      const long m = ((long)(a + n / 2) * (2 * u + N + 1)) % (2L * N);
-      const double ang = -M_PI * (double)m / (double)N;
-      hd[u * n + a] = make_double2(cos(ang), sin(ang));
-      h[u * n + a] = make_float2((float)cos(ang), (float)sin(ang));
-    }
-  // synchronous on purpose: `h` is a stack buffer; happens once per (device, n)
-  cudaError_t e = cudaMemcpyToSymbol(c_tw, h, sizeof(float2) * N * n);
-  if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_twd, hd, sizeof(double2) * N * n);
-  if (e != cudaSuccess) return fail(-3, "twiddle upload: %s", cudaGetErrorString(e));
-  if (dev < 64) g_tw_n[dev] = n;
-  (void)stream;
-  return 0;
-}
 
 // ---- per-pixel random stream: Philox counter = (pixel, env, frame_lo, frame_hi16 << 16 | block) -------------------
 // Block 0 of a pixel's stream feeds the photon draw (words x, y) and the read-out normal (z, w); block 1 the dark
@@ -74,6 +48,48 @@ constexpr RcpTable make_rcp() {
   return t;
 }
 __constant__ RcpTable c_rcp_table = make_rcp();
+
+// n = 10, 12: only the float64 calibration kernel reads a table (their spots kernel uses literal twiddles), so they get a
+// float64 table of their own, declared after the tables the n <= 8 kernels read so that those kernels' constant-bank
+// offsets do not move
+constexpr int kMaxWideN = 12;
+__constant__ double2 c_twd_wide[2 * kMaxWideN * kMaxWideN];
+template <int n>
+__device__ __forceinline__ double2 twd(int i) {
+  if constexpr (n <= kMaxN) return c_twd[i];
+  else return c_twd_wide[i];
+}
+static int g_tw_n[64] = {0};             // per device: n for which c_tw / c_twd (c_twd_wide) are currently valid
+static std::mutex g_tw_mutex;
+
+static int ensure_twiddles(int n, cudaStream_t stream) {
+  int dev = 0;
+  cudaGetDevice(&dev);
+  std::lock_guard<std::mutex> lock(g_tw_mutex);
+  if (dev < 64 && g_tw_n[dev] == n) return 0;
+  const int N = 2 * n;
+  float2 h[2 * kMaxWideN * kMaxWideN];
+  double2 hd[2 * kMaxWideN * kMaxWideN];
+  for (int u = 0; u < N; ++u)
+    for (int a = 0; a < n; ++a) {
+      const long m = ((long)(a + n / 2) * (2 * u + N + 1)) % (2L * N);
+      const double ang = -M_PI * (double)m / (double)N;
+      hd[u * n + a] = make_double2(cos(ang), sin(ang));
+      h[u * n + a] = make_float2((float)cos(ang), (float)sin(ang));
+    }
+  // synchronous on purpose: `h` is a stack buffer; happens once per (device, n)
+  cudaError_t e = cudaSuccess;
+  if (n <= kMaxN) {
+    e = cudaMemcpyToSymbol(c_tw, h, sizeof(float2) * N * n);
+    if (e == cudaSuccess) e = cudaMemcpyToSymbol(c_twd, hd, sizeof(double2) * N * n);
+  } else {
+    e = cudaMemcpyToSymbol(c_twd_wide, hd, sizeof(double2) * N * n);
+  }
+  if (e != cudaSuccess) return fail(-3, "twiddle upload: %s", cudaGetErrorString(e));
+  if (dev < 64) g_tw_n[dev] = n;
+  (void)stream;
+  return 0;
+}
 
 // Poisson(lambda), lambda < 12, by inversion of the uniform u in (0, 1): sequential search from k = 0.  The first
 // sixteen terms are unrolled with literal reciprocals (four FP32 instructions and a branch per term, no table load); the
@@ -1016,8 +1032,214 @@ shwfs_frame_split_kernel(const float* __restrict__ opd_a, const float* __restric
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// n = 10, 12 (the spots kernel of the wide lenslets, both in aoenv_shwfs_frame and in aoenv_shwfs_frame_dm): the arithmetic
+// of shwfs_frame_kernel — radix-2 split of both pruned DFT passes, packed FP32, literal twiddles — on T = n / 2 lanes per
+// lenslet.  One thread per lenslet would hold the 2 n^2 floats of the field next to the pass-2 rows and accumulators
+// (~360 live floats at n = 12).  Lane t owns tile rows 2t, 2t+1 (= the column pair (2t, 2t+1) of the
+// transposed field): it loads those 2n pixels, evaluates their DM surface in place (WL > 0, the same operations in the
+// same order as shwfs_frame_kernel<n, WL>), accumulates the pupil statistics and forms the field.  Then two rounds, one per
+// parity du of the output row: every lane runs pass 1 of its column pair for the rows u = 2p + du (p < T), the lanes of
+// a lenslet swap those rows through a warp-private patch of shared memory (__syncwarp, no block barrier), and lane p runs
+// pass 2 of row u = 2p + du (and u + n), |.|^2 and the binning into binned rows p and p + n/2.  Splitting by du halves the
+// patch (27 KB per 128-thread CTA at n = 12 instead of 55 KB) at no cost in arithmetic.  `order` (nullable) visits the
+// lenslets lit-first, as in shwfs_frame_kernel.
+// ---------------------------------------------------------------------------------------------------------
+template <int n, int WL>
+__global__ void __launch_bounds__(128, n == 12 ? 3 : 4)      // n = 12: 168 registers, no spills (at 128 it spills)
+shwfs_frame_wide_kernel(const float* __restrict__ opd_a, const float* __restrict__ opd_b, const float* __restrict__ pupil,
+                        const float* __restrict__ amp, const uint8_t* __restrict__ valid, int nS, float phase_scale,
+                        int track_max, int shared_max, float* __restrict__ frame, int32_t* __restrict__ envmax,
+                        double* __restrict__ stats, const __grid_constant__ aoenv_dm_sep_t dm, const int32_t* __restrict__ order) {
+  constexpr int N = 2 * n, T = n / 2, h = n / 2, LPW = 32 / T, S = LPW + 1;
+  // exchange of one round: [warp][(kind * T + source lane) * T + destination lane][slot] float2, kind = Pr, Pi, Qr, Qi
+  __shared__ float2 xch[4][4 * T * T][S];
+  pdl_enter();
+  const int R = nS * n;
+  const int b = blockIdx.y;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int slot = lane / T, t = lane - slot * T;
+  const int k0 = (blockIdx.x * 4 + warp) * LPW + slot;
+  const bool active = slot < LPW && k0 < nS * nS;
+  const int k = (active && order != nullptr) ? __ldg(&order[k0]) : k0;
+  const int li = active ? k / nS : 0, lj = active ? k - li * nS : 0;
+  const bool lit = active && valid[k] != 0;
+  const float phase_turns = phase_scale * 0.15915494309189535f;
+  const size_t tile = (size_t)(li * n) * R + lj * n;
+  float f0 = 0.f, f1 = 0.f, f2 = 0.f, f3 = 0.f;                         // pupil statistics, see shwfs_frame_kernel
+  float2 er2[n], ei2[n];                                                  // (E[a][2t], E[a][2t+1])
+  if (active) {
+    const float* __restrict__ pa = opd_a + (size_t)b * R * R + tile;
+    const float* __restrict__ pb = (WL == 0 && opd_b) ? opd_b + (size_t)b * R * R + tile : nullptr;
+    const size_t centre = (size_t)b * R * R + (size_t)(R / 2) * R + R / 2;
+    const float ka = stats ? __ldg(opd_a + centre) : 0.f;
+    // (with the in-place DM the total is centred on the atmosphere's centre value, as in shwfs_frame_kernel)
+    const float kt = stats ? (pb ? ka + __ldg(opd_b + centre) : ka) : 0.f;
+    // DM surface of tile rows 2t + e: dmv[e][a2] = pixels (columns 2 a2, 2 a2 + 1)
+    float2 dmv[2][WL > 0 ? h : 1];
+    if constexpr (WL > 0) {
+      constexpr int half = (WL + 1) / 2, hp = (half + 3) / 4 * 4;
+#pragma unroll
+      for (int e = 0; e < 2; ++e)
+#pragma unroll
+        for (int a2 = 0; a2 < h; ++a2) dmv[e][a2] = make_float2(0.f, 0.f);
+      const float* __restrict__ trow = dm.rows + ((size_t)b * dm.nActP + __ldg(&dm.ilr[li])) * R + lj * n;
+      const float* __restrict__ wrow = dm.wlr + (size_t)(li * n + 2 * t) * (2 * hp);
+#pragma unroll
+      for (int g = 0; g < 2 * hp / 4; ++g) {
+        float4 w4[2];
+#pragma unroll
+        for (int e = 0; e < 2; ++e) w4[e] = __ldg(reinterpret_cast<const float4*>(wrow + (size_t)e * (2 * hp)) + g);
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const int j = 4 * g + c, hh = j / hp, kk = j % hp;
+          if (kk >= half) continue;                      // padding entries of the weight rows
+          const int tr = hh * half + kk;
+          if (tr >= WL) continue;
+          float2 tv[h];
+#pragma unroll
+          for (int a2 = 0; a2 < h; ++a2) tv[a2] = __ldg(reinterpret_cast<const float2*>(trow + (size_t)tr * R) + a2);
+#pragma unroll
+          for (int e = 0; e < 2; ++e) {
+            const float w = c == 0 ? w4[e].x : (c == 1 ? w4[e].y : (c == 2 ? w4[e].z : w4[e].w));
+#pragma unroll
+            for (int a2 = 0; a2 < h; ++a2) dmv[e][a2] = fma2(dup2(w), tv[a2], dmv[e][a2]);
+          }
+        }
+      }
+    }
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      const int bb = 2 * t + e;
+#pragma unroll
+      for (int a2 = 0; a2 < h; ++a2) {
+        const int o2 = bb * R + 2 * a2;
+        const float2 av = __ldg(reinterpret_cast<const float2*>(pa + o2));
+        float2 bv;
+        if constexpr (WL > 0) bv = dmv[e][a2];
+        else bv = pb ? __ldg(reinterpret_cast<const float2*>(pb + o2)) : make_float2(0.f, 0.f);
+        const float2 pv = __ldg(reinterpret_cast<const float2*>(pupil + tile + o2));
+        const float2 mv = lit ? __ldg(reinterpret_cast<const float2*>(amp + tile + o2)) : make_float2(0.f, 0.f);
+#pragma unroll
+        for (int h2 = 0; h2 < 2; ++h2) {
+          const int aa = 2 * a2 + h2;
+          const float a = h2 ? av.y : av.x;
+          const float tt = a + (h2 ? bv.y : bv.x);
+          const float pu = h2 ? pv.y : pv.x;
+          const float in_pupil = pu > 0.f ? 1.f : 0.f;
+          const float da = (a - ka) * in_pupil, dt = (tt - kt) * in_pupil;
+          f0 += da; f1 = fmaf(da, da, f1); f2 += dt; f3 = fmaf(dt, dt, f3);
+          const float turns = tt * pu * phase_turns;
+          const float ang = (turns - ((turns + 12582912.0f) - 12582912.0f)) * 6.283185307179586f;
+          const float am = h2 ? mv.y : mv.x;
+          const float cs = am * __cosf(ang), sn = am * __sinf(ang);
+          if (e == 0) { er2[aa].x = cs; ei2[aa].x = sn; } else { er2[aa].y = cs; ei2[aa].y = sn; }
+        }
+      }
+    }
+  }
+  if (stats != nullptr) {       // one atomic per warp and statistic
+    double s0 = warp_sum((double)f0), s1 = warp_sum((double)f1), s2 = warp_sum((double)f2), s3 = warp_sum((double)f3);
+    if (lane == 0) {
+      double* __restrict__ st = stats + (size_t)b * 4;
+      atomicAdd(st, s0); atomicAdd(st + 1, s1); atomicAdd(st + 2, s2); atomicAdd(st + 3, s3);
+    }
+  }
+  float2 (*x)[S] = xch[warp];
+  const bool any_lit = __any_sync(0xffffffffu, lit);
+  float vmax = -INFINITY;
+  if (any_lit) {                                                          // warp-uniform: every lane meets the __syncwarps
+    float2 acc[n];                         // acc[q] = (binned row t, binned row t + n/2) at binned column q
+#pragma unroll
+    for (int q = 0; q < n; ++q) acc[q] = make_float2(0.f, 0.f);
+#pragma unroll
+    for (int du = 0; du < 2; ++du) {
+      if (lit) {
+        // pass 1 for this lane's column pair, output rows u = 2p + du (rows u + n follow by the radix-2 symmetry)
+#pragma unroll
+        for (int p = 0; p < T; ++p) {
+          const int u = 2 * p + du;
+          float2 pr = make_float2(0.f, 0.f), pi = pr, qr = pr, qi = pr;
+#pragma unroll
+          for (int aa = 0; aa < n; ++aa) {
+            const float gx = WfsTw<n>::re(u * n + aa), gy = WfsTw<n>::im(u * n + aa);
+            if (((aa + h) & 1) == 0) {
+              pr = fma2(dup2(gx), er2[aa], fma2(dup2(-gy), ei2[aa], pr));
+              pi = fma2(dup2(gx), ei2[aa], fma2(dup2(gy), er2[aa], pi));
+            } else {
+              qr = fma2(dup2(gx), er2[aa], fma2(dup2(-gy), ei2[aa], qr));
+              qi = fma2(dup2(gx), ei2[aa], fma2(dup2(gy), er2[aa], qi));
+            }
+          }
+          x[(0 * T + t) * T + p][slot] = pr;
+          x[(1 * T + t) * T + p][slot] = pi;
+          x[(2 * T + t) * T + p][slot] = qr;
+          x[(3 * T + t) * T + p][slot] = qi;
+        }
+      }
+      __syncwarp();
+      if (lit) {
+        float2 yr[n], yi[n];                 // (row u: P + Q, row u + n: P - Q), u = 2t + du
+#pragma unroll
+        for (int kk = 0; kk < T; ++kk) {
+          const float2 pr = x[(0 * T + kk) * T + t][slot], pi = x[(1 * T + kk) * T + t][slot];
+          const float2 qr = x[(2 * T + kk) * T + t][slot], qi = x[(3 * T + kk) * T + t][slot];
+          yr[2 * kk] = make_float2(pr.x + qr.x, pr.x - qr.x);
+          yr[2 * kk + 1] = make_float2(pr.y + qr.y, pr.y - qr.y);
+          yi[2 * kk] = make_float2(pi.x + qi.x, pi.x - qi.x);
+          yi[2 * kk + 1] = make_float2(pi.y + qi.y, pi.y - qi.y);
+        }
+#pragma unroll
+        for (int v = 0; v < n; ++v) {
+          float2 er_ = make_float2(0.f, 0.f), ei_ = er_, or_ = er_, oi_ = er_;
+#pragma unroll
+          for (int bb = 0; bb < n; ++bb) {
+            const float gx = WfsTw<n>::re(v * n + bb), gy = WfsTw<n>::im(v * n + bb);
+            if (((bb + h) & 1) == 0) {
+              er_ = fma2(yr[bb], dup2(gx), fma2(yi[bb], dup2(-gy), er_));
+              ei_ = fma2(yr[bb], dup2(gy), fma2(yi[bb], dup2(gx), ei_));
+            } else {
+              or_ = fma2(yr[bb], dup2(gx), fma2(yi[bb], dup2(-gy), or_));
+              oi_ = fma2(yr[bb], dup2(gy), fma2(yi[bb], dup2(gx), oi_));
+            }
+          }
+          const float2 f0r = add2(er_, or_), f0i = add2(ei_, oi_);     // F[row][v]
+          const float2 f1r = sub2(er_, or_), f1i = sub2(ei_, oi_);     // F[row][v + n]
+          acc[v >> 1] = add2(acc[v >> 1], fma2(f0r, f0r, mul2(f0i, f0i)));
+          acc[(v >> 1) + h] = add2(acc[(v >> 1) + h], fma2(f1r, f1r, mul2(f1i, f1i)));
+        }
+      }
+      __syncwarp();                                                       // the patch is rewritten by the next round
+    }
+    if (lit) {
+      float* __restrict__ fout = frame + (size_t)b * R * R + tile;
+      const float norm = 1.0f / (float)(N * N);
+#pragma unroll
+      for (int q2 = 0; q2 < h; ++q2) {
+        const float2 lo = make_float2(acc[2 * q2].x * norm, acc[2 * q2 + 1].x * norm);
+        const float2 hi = make_float2(acc[2 * q2].y * norm, acc[2 * q2 + 1].y * norm);
+        *reinterpret_cast<float2*>(fout + (size_t)t * R + 2 * q2) = lo;
+        *reinterpret_cast<float2*>(fout + (size_t)(t + h) * R + 2 * q2) = hi;
+        vmax = fmaxf(vmax, fmaxf(fmaxf(lo.x, lo.y), fmaxf(hi.x, hi.y)));
+      }
+    }
+  }
+  if (active && !lit) {                                                   // dark lenslet: rows 2t, 2t+1 of its tile
+    float* __restrict__ fout = frame + (size_t)b * R * R + tile;
+#pragma unroll
+    for (int e = 0; e < 2; ++e)
+#pragma unroll
+      for (int q2 = 0; q2 < h; ++q2) *reinterpret_cast<float2*>(fout + (size_t)(2 * t + e) * R + 2 * q2) = make_float2(0.f, 0.f);
+  }
+  if (track_max) {            // with a camera model the maximum is taken after the detector pass
+    vmax = warp_max(vmax);
+    if (lane == 0 && vmax > -INFINITY) atomicMax(&envmax[shared_max ? 0 : b], float_to_ordered(vmax));
+  }
+}
+
 // centroid + slopes: one thread per (valid lenslet, environment).  n is a template parameter so that the 6 x 6 (4 x 4,
-// 8 x 8) spot is read with fully unrolled 64-bit loads (tile rows start on even columns: lj * n with n even).
+// 8 x 8, 10 x 10, 12 x 12) spot is read with fully unrolled 64-bit loads (tile rows start on even columns: lj * n with n
+// even).
 template <int n>
 __global__ void __launch_bounds__(128)
 shwfs_slopes_kernel(const float* __restrict__ frame, const int32_t* __restrict__ envmax, int shared_max,
@@ -1112,7 +1334,7 @@ shwfs_frame_f64_kernel(const float* __restrict__ opd, const float* __restrict__ 
       for (int bb = 0; bb < n; ++bb) { yr[bb] = 0.0; yi[bb] = 0.0; }
 #pragma unroll
       for (int aa = 0; aa < n; ++aa) {
-        const double2 g = c_twd[u * n + aa];
+        const double2 g = twd<n>(u * n + aa);
 #pragma unroll
         for (int bb = 0; bb < n; ++bb) {
           yr[bb] += g.x * er[aa][bb] - g.y * ei[aa][bb];
@@ -1124,7 +1346,7 @@ shwfs_frame_f64_kernel(const float* __restrict__ opd, const float* __restrict__ 
         double fr = 0.0, fi = 0.0;
 #pragma unroll
         for (int bb = 0; bb < n; ++bb) {
-          const double2 g = c_twd[v * n + bb];
+          const double2 g = twd<n>(v * n + bb);
           fr += yr[bb] * g.x - yi[bb] * g.y;
           fi += yr[bb] * g.y + yi[bb] * g.x;
         }
@@ -1217,7 +1439,12 @@ static int shwfs_frame_impl(const float* opd_a, const float* opd_b, const aoenv_
     AOENV_CHECK_ARG((reinterpret_cast<uintptr_t>(dm.rows) & 7) == 0 && (reinterpret_cast<uintptr_t>(dm.wlr) & 15) == 0,
                     "shwfs_frame_dm: DM tables must be 16-byte aligned");
   }
-  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8, "shwfs_frame: %d pixels per lenslet is not a compiled size (4, 6, 8)", n);
+  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8 || n == 10 || n == 12,
+                  "shwfs_frame: %d pixels per lenslet is not a compiled size (4, 6, 8, 10, 12)", n);
+  const int variant = g_wfs6_factorised.load(std::memory_order_relaxed);
+  AOENV_CHECK_ARG(n <= 8 || variant == 0,
+                  "shwfs_frame: the alternative frame variant %d (aoenv_set_wfs6_variant / AOENV_WFS_FRAME) is compiled for "
+                  "4, 6, 8 pixels per lenslet, not %d", variant, n);
   cudaStream_t s = (cudaStream_t)stream;
   if (det) {
     AOENV_CHECK_ARG(!(det->bits > 0 && !det->has_fwc), "shwfs_frame: ADC without a full-well capacity is not supported");
@@ -1228,8 +1455,23 @@ static int shwfs_frame_impl(const float* opd_a, const float* opd_b, const aoenv_
   AOENV_LAUNCH(envmax_init_kernel, dim3((4 * B + 255) / 256), 256, 0, s, envmax, shared_max ? 1 : B, stats, stats ? 4 * B : 0);
   AOENV_LAUNCH_CHECK("envmax_init");
   dim3 grid((nS * nS + 127) / 128, B);
-  const int variant = g_wfs6_factorised.load(std::memory_order_relaxed);
-  if (variant == 3 && dm.WL == 0) {            // n / 2 lanes per lenslet, any compiled n
+  if (n > 8) {                                 // n / 2 lanes per lenslet, 4 warps per CTA
+    const int per_block = 4 * (32 / (n / 2));
+    dim3 gw((nS * nS + per_block - 1) / per_block, B);
+#define AOENV_WFS_WIDE(NN, WW)                                                                                            \
+  AOENV_LAUNCH((shwfs_frame_wide_kernel<NN, WW>), gw, 128, 0, s, opd_a, opd_b, pupil, amp, valid, nS, phase_scale,        \
+               (int)(det == nullptr), shared_max, frame, envmax, stats, dm, order)
+    if (n == 10) {
+      if (dm.WL == 14) AOENV_WFS_WIDE(10, 14);
+      else if (dm.WL == 18) AOENV_WFS_WIDE(10, 18);
+      else AOENV_WFS_WIDE(10, 0);
+    } else {
+      if (dm.WL == 14) AOENV_WFS_WIDE(12, 14);
+      else if (dm.WL == 18) AOENV_WFS_WIDE(12, 18);
+      else AOENV_WFS_WIDE(12, 0);
+    }
+#undef AOENV_WFS_WIDE
+  } else if (variant == 3 && dm.WL == 0) {     // n / 2 lanes per lenslet, any compiled n
     const int per_block = 4 * (32 / (n / 2));
     dim3 g3((nS * nS + per_block - 1) / per_block, B);
     if (n == 4) shwfs_frame_split_kernel<4><<<g3, 128, 0, s>>>(opd_a, opd_b, pupil, amp, valid, nS, phase_scale, det == nullptr, shared_max, frame, envmax, stats);
@@ -1330,7 +1572,8 @@ int aoenv_shwfs_slopes(const float* frame, const int32_t* envmax, int shared_max
                        const float* ref_xy, float inv_units, float threshold_cog, int B, int nS, int n, float* slopes,
                        int lds, void* slope_planes, int parts, void* stream) {
   AOENV_CHECK_ARG(B > 0 && B <= 65535 && nV > 0 && lds >= 2 * nV, "shwfs_slopes: bad shape B=%d nV=%d lds=%d", B, nV, lds);
-  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8, "shwfs_slopes: %d pixels per lenslet is not a compiled size (4, 6, 8)", n);
+  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8 || n == 10 || n == 12,
+                  "shwfs_slopes: %d pixels per lenslet is not a compiled size (4, 6, 8, 10, 12)", n);
   AOENV_CHECK_ARG((reinterpret_cast<uintptr_t>(frame) & 7) == 0, "shwfs_slopes: frame must be 8-byte aligned");
   dim3 grid((nV + 127) / 128, B);
 #define AOENV_SLOPES_CASE(NN)                                                                                          \
@@ -1342,6 +1585,8 @@ int aoenv_shwfs_slopes(const float* frame, const int32_t* envmax, int shared_max
     AOENV_SLOPES_CASE(4)
     AOENV_SLOPES_CASE(6)
     AOENV_SLOPES_CASE(8)
+    AOENV_SLOPES_CASE(10)
+    AOENV_SLOPES_CASE(12)
   }
 #undef AOENV_SLOPES_CASE
   AOENV_LAUNCH_CHECK("shwfs_slopes");
@@ -1353,7 +1598,8 @@ int aoenv_shwfs_measure_f64(const float* opd, const float* pupil, const float* a
                             int F, int nS, int n, double phase_scale, int shared_max, double* frame, uint64_t* envmax,
                             double* slopes, int lds, void* stream) {
   AOENV_CHECK_ARG(F > 0 && F <= 65535 && nS > 0 && nV > 0 && lds >= 2 * nV, "shwfs_measure_f64: bad shape");
-  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8, "shwfs_measure_f64: %d pixels per lenslet is not a compiled size (4, 6, 8)", n);
+  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8 || n == 10 || n == 12,
+                  "shwfs_measure_f64: %d pixels per lenslet is not a compiled size (4, 6, 8, 10, 12)", n);
   cudaStream_t s = (cudaStream_t)stream;
   int rc = ensure_twiddles(n, s);
   if (rc) return rc;
@@ -1365,6 +1611,8 @@ int aoenv_shwfs_measure_f64(const float* opd, const float* pupil, const float* a
     case 4: shwfs_frame_f64_kernel<4><<<grid, 64, 0, s>>>(opd, pupil, amp, valid, nS, phase_scale, shared_max, frame, em); break;
     case 6: shwfs_frame_f64_kernel<6><<<grid, 64, 0, s>>>(opd, pupil, amp, valid, nS, phase_scale, shared_max, frame, em); break;
     case 8: shwfs_frame_f64_kernel<8><<<grid, 64, 0, s>>>(opd, pupil, amp, valid, nS, phase_scale, shared_max, frame, em); break;
+    case 10: shwfs_frame_f64_kernel<10><<<grid, 64, 0, s>>>(opd, pupil, amp, valid, nS, phase_scale, shared_max, frame, em); break;
+    case 12: shwfs_frame_f64_kernel<12><<<grid, 64, 0, s>>>(opd, pupil, amp, valid, nS, phase_scale, shared_max, frame, em); break;
   }
   AOENV_LAUNCH_CHECK("shwfs_frame_f64");
   dim3 g2((nV + 127) / 128, F);

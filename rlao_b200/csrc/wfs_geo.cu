@@ -275,7 +275,8 @@ int aoenv_shwfs_geometric(const float* opd_a, const float* opd_b, const aoenv_dm
                           float inv_units, float* slopes, int lds, void* slope_planes, int parts, double* stats, void* stream) {
   AOENV_CHECK_ARG(B > 0 && B <= 65535 && nS > 0 && nV > 0 && lds >= 2 * nV, "shwfs_geometric: bad shape B=%d nS=%d nV=%d lds=%d",
                   B, nS, nV, lds);
-  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8, "shwfs_geometric: %d pixels per lenslet is not a compiled size (4, 6, 8)", n);
+  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8 || n == 10 || n == 12,
+                  "shwfs_geometric: %d pixels per lenslet is not a compiled size (4, 6, 8, 10, 12)", n);
   AOENV_CHECK_ARG(opd_a != nullptr && pupil != nullptr && flux != nullptr && valid_idx != nullptr && slopes != nullptr,
                   "shwfs_geometric: null argument");
   AOENV_CHECK_ARG(slope_planes == nullptr || parts == 2 || parts == 3, "shwfs_geometric: parts=%d", parts);
@@ -311,7 +312,9 @@ int aoenv_shwfs_geometric(const float* opd_a, const float* opd_b, const aoenv_dm
   switch (n) {
     case 4: rc = dispatch_v<4>(V, dm.WL, grid, smem, s, opd_a, opd_b, dm, pupil, flux, valid_idx, nV, nS, SL, scale, slopes, lds, planes, parts, stats); break;
     case 6: rc = dispatch_v<6>(V, dm.WL, grid, smem, s, opd_a, opd_b, dm, pupil, flux, valid_idx, nV, nS, SL, scale, slopes, lds, planes, parts, stats); break;
-    default: rc = dispatch_v<8>(V, dm.WL, grid, smem, s, opd_a, opd_b, dm, pupil, flux, valid_idx, nV, nS, SL, scale, slopes, lds, planes, parts, stats); break;
+    case 8: rc = dispatch_v<8>(V, dm.WL, grid, smem, s, opd_a, opd_b, dm, pupil, flux, valid_idx, nV, nS, SL, scale, slopes, lds, planes, parts, stats); break;
+    case 10: rc = dispatch_v<10>(V, dm.WL, grid, smem, s, opd_a, opd_b, dm, pupil, flux, valid_idx, nV, nS, SL, scale, slopes, lds, planes, parts, stats); break;
+    default: rc = dispatch_v<12>(V, dm.WL, grid, smem, s, opd_a, opd_b, dm, pupil, flux, valid_idx, nV, nS, SL, scale, slopes, lds, planes, parts, stats); break;
   }
   if (rc) return rc;
   AOENV_LAUNCH_CHECK("shwfs_geometric");
@@ -321,7 +324,8 @@ int aoenv_shwfs_geometric(const float* opd_a, const float* opd_b, const aoenv_dm
 int aoenv_shwfs_geometric_f64(const float* opd, const float* flux, const int32_t* valid_idx, int nV, int F, int nS, int n,
                               double phase_scale, double inv_units, double* slopes, int lds, void* stream) {
   AOENV_CHECK_ARG(F > 0 && F <= 65535 && nS > 0 && nV > 0 && lds >= 2 * nV, "shwfs_geometric_f64: bad shape");
-  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8, "shwfs_geometric_f64: %d pixels per lenslet is not a compiled size (4, 6, 8)", n);
+  AOENV_CHECK_ARG(n == 4 || n == 6 || n == 8 || n == 10 || n == 12,
+                  "shwfs_geometric_f64: %d pixels per lenslet is not a compiled size (4, 6, 8, 10, 12)", n);
   AOENV_CHECK_ARG(opd != nullptr && flux != nullptr && valid_idx != nullptr && slopes != nullptr, "shwfs_geometric_f64: null argument");
   cudaStream_t s = (cudaStream_t)stream;
   dim3 grid((nV + 127) / 128, F);
@@ -329,7 +333,9 @@ int aoenv_shwfs_geometric_f64(const float* opd, const float* flux, const int32_t
   switch (n) {
     case 4: shwfs_geometric_f64_kernel<4><<<grid, 128, 0, s>>>(opd, flux, valid_idx, nV, nS, scale, slopes, lds); break;
     case 6: shwfs_geometric_f64_kernel<6><<<grid, 128, 0, s>>>(opd, flux, valid_idx, nV, nS, scale, slopes, lds); break;
-    default: shwfs_geometric_f64_kernel<8><<<grid, 128, 0, s>>>(opd, flux, valid_idx, nV, nS, scale, slopes, lds); break;
+    case 8: shwfs_geometric_f64_kernel<8><<<grid, 128, 0, s>>>(opd, flux, valid_idx, nV, nS, scale, slopes, lds); break;
+    case 10: shwfs_geometric_f64_kernel<10><<<grid, 128, 0, s>>>(opd, flux, valid_idx, nV, nS, scale, slopes, lds); break;
+    default: shwfs_geometric_f64_kernel<12><<<grid, 128, 0, s>>>(opd, flux, valid_idx, nV, nS, scale, slopes, lds); break;
   }
   AOENV_LAUNCH_CHECK("shwfs_geometric_f64");
   return 0;
