@@ -33,7 +33,8 @@ __device__ __forceinline__ void store_vec(float* p, const float (&v)[V]) {
 // operations in the same order as shwfs_frame_kernel: the surface is bit-identical to the one the frame kernel sees.
 // Then one thread per lenslet sums its n x n pixels in row-major order — weighted gradients, weights, and the four pupil
 // statistics in float32 exactly as the frame kernel does per lenslet — so slopes need no atomics and the statistics equal
-// the frame kernel's up to the order of the float64 reduction.
+// the frame kernel's up to the order of the float64 reduction (at 4 to 8 pixels; the wide frame kernel of 10 and 12 pixels
+// splits a lenslet over n / 2 lanes and adds its float32 partial sums in another order: agreement to float32 rounding).
 template <int n, int V, int WL>
 __global__ void __launch_bounds__(kGeoThreads)
 shwfs_geometric_kernel(const float* __restrict__ opd_a, const float* __restrict__ opd_b, const __grid_constant__ aoenv_dm_sep_t dm,

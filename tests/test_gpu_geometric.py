@@ -17,6 +17,15 @@ pytestmark = pytest.mark.gpu
 
 SLOPE_TOL = 1e-4
 STATS_TOL = 1e-9
+# Lenslets of 10 and 12 pixels: the wide frame kernel splits a lenslet over n / 2 lanes and adds its float32 partial sums
+# in another order than the geometric kernel's one thread per lenslet; the statistics then agree to float32 rounding only
+# (measured 2e-8 to 5e-8 on B200)
+WIDE_STATS_TOL = 5e-7
+
+
+def stats_tol(n):
+    """Tolerance of the geometric kernel's pupil statistics against the frame kernel's at n pixels per lenslet."""
+    return STATS_TOL if n <= 8 else WIDE_STATS_TOL
 
 
 @pytest.fixture(scope="module")
@@ -56,8 +65,9 @@ def _frame_stats(wfs, opd_a, opd_b=None, dm=None):
     return _np(stats)
 
 
-@pytest.mark.parametrize("nS", [8, 20, 40])
-@pytest.mark.parametrize("n", [4, 6, 8])
+# (n, nS): every lenslet size of 4-8 pixels at 8, 20 and 40 lenslets, and two odd pupils of R = 2 (mod 4) pixels (the
+# float2 kernels): 7 x 6 and 5 x 10
+@pytest.mark.parametrize("n,nS", [(n, nS) for n in (4, 6, 8) for nS in (8, 20, 40)] + [(6, 7), (10, 5)])
 def test_geometric_kernels_vs_oracle(dev, nS, n):
     from rlao_b200.ShackHartmann import ShackHartmann
     from rlao_b200.Source import Source
@@ -93,7 +103,7 @@ def test_geometric_kernels_vs_oracle(dev, nS, n):
     got = _np(slopes)[:, :wfs.nSignal]
     for e in range(B):
         assert rel_err(got[e], orc.measure(tot[e] * 2 * np.pi / wl)) < SLOPE_TOL, (e, "slopes, two terms")
-    assert rel_err(_np(stats), _frame_stats(wfs, a, b)) < STATS_TOL
+    assert rel_err(_np(stats), _frame_stats(wfs, a, b)) < stats_tol(n)
     # calibration-grade twin (multi-frame branch)
     frames = wfs.measure_frames(a) * wfs.slopes_units
     want = orc.measure_multi(a32.astype(np.float64) * 2 * np.pi / wl).T * orc.slopes_units

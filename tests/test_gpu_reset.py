@@ -27,7 +27,7 @@ def _synth_screens(synth, S, seed=1, screen0=0, inject=None):
     return out
 
 
-@pytest.mark.parametrize("R", [48, 120, 240])
+@pytest.mark.parametrize("R", [42, 48, 120, 240])          # (N = R + 4: 46 = 2 mod 4, the others 0 mod 4)
 def test_screens_from_injected_draws_equal_the_reference_algorithm(dev, R):
     """The reference draws normal(size=(N,N)) twice from RandomState(seed) (real, imaginary parts) and reuses the head of the
     same stream for the sub-harmonics; fed with those draws the device path must reproduce its screens."""
